@@ -19,6 +19,14 @@ GPU (frame-sharded across GPUs, weak scaling, no data-path collective: frames ar
   cpu_baseline  the unmodified reference CPU backend (oracle/_ref) on a bounded row sample
 
 `--impl reference` times the reference's own CPU implementation on the host cores instead.
+
+`--dump-outputs DIR` writes what the timed path returned in its last step, so that two builds can be compared
+output for output: disparity_<f>.npy and corrmap_<f>.npy (float32, [DUMP_ROWS, 2048]) for every frame f of
+rank 0, on the same rows of every frame, drawn once with a fixed seed. The library marks invalid disparities
+and corrmap cells it never evaluated as NaN; the dump keeps every value finite: such cells are written as 0 and
+disparity_valid_<f>.npy / corrmap_valid_<f>.npy (float32, 1 = a number, 0 = NaN) say which they are (48 MiB in
+all). The frames are a pure function of their index (libbicos_b200/synth.py), so the same arguments give the
+same inputs in every run.
 """
 
 import argparse
@@ -51,6 +59,24 @@ CONFIG = {
     "l2": f"inputs larger than L2 ({FRAMES} x 208 MB per GPU per step); no explicit flush",
     "reference_arm_sample": "a bounded row sample of one stereo stack per step (cost is linear in rows), see cpu_baseline.sample",
 }
+DUMP_ROWS, DUMP_SEED = 384, 20261020
+
+
+def dump_outputs(directory, outs):
+    """--dump-outputs: the (disparity, corrmap) pairs of one step, on a fixed seeded sample of rows; NaN cells as 0
+    beside a float validity mask, so that every value written is finite."""
+    import numpy as np
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(ROWS, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(outs[0][0].device)
+    for f, (disp, corr) in enumerate(outs):
+        for name, a in (("disparity", disp), ("corrmap", corr)):
+            a = a.index_select(0, idx)
+            valid = torch.isfinite(a)
+            np.save(os.path.join(directory, f"{name}_{f}.npy"), torch.where(valid, a, torch.zeros_like(a)).cpu().numpy())
+            np.save(os.path.join(directory, f"{name}_valid_{f}.npy"), valid.to(a.dtype).cpu().numpy())
 
 
 def load_peaks():
@@ -258,7 +284,14 @@ def main():
     ap.add_argument("--table", action="store_true",
                     help="instead of the bench line: every BASELINE config (tools/bench_configs.py) with the "
                          "reference's CUDA backend timed beside it, one JSON line per config")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the disparity and corrmap of the last step's frames to "
+                         "DIR/<name>.npy (float32, a fixed seeded sample of rows; NaN cells as 0 beside validity masks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.table):
+        ap.error("--dump-outputs dumps the timed path of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -354,6 +387,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     # frame 0 as the timed region left it (the engine comparison further down writes into `outs` again)
     timed_frame0 = (outs[0][0].cpu().numpy(), outs[0][1].cpu().numpy()) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)
     ms_per_step = total_ms / args.steps
     value = world * FRAMES * px / (ms_per_step * 1e-3) / 1e6
 

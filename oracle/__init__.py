@@ -6,13 +6,15 @@ is CUDA-only and fails loudly without its extension.
 
 Two checkers, same Python surface:
 
-* ``oracle.ref``  -- the UNMODIFIED reference CPU backend (/root/reference/src/impl/cpu.cpp
+* ``oracle.ref``  -- the UNMODIFIED reference CPU backend (<REFERENCE_DIR>/src/impl/cpu.cpp
   and friends) compiled against oracle/shim into oracle/_ref/libbicos_ref.so by
-  oracle/Makefile. Present in the build container (and travels to the GPU box as a
-  prebuilt .so); ``oracle.ref.available()`` says whether it can be loaded.
+  oracle/Makefile when BICOS_REFERENCE_DIR names a checkout of the reference project (a prebuilt
+  oracle/_ref is kept otherwise); ``oracle.ref.available()`` says whether it can be loaded.
 * ``oracle.port`` -- oracle/bicos_oracle.c, a plain-C restatement of the same algorithm
   (each function cites the reference file:line it follows). Pinned against ``oracle.ref``
-  and against tests/golden/*.npz (generated from ``oracle.ref`` by tests/golden/make_golden.py).
+  and against tests/golden/*.npz (generated from ``oracle.ref`` by tests/golden/make_golden.py); without the
+  reference build, the tests that compare with it use the outputs stored under tests/golden/reference/
+  (tests/golden/make_reference_outputs.py).
 """
 
 from __future__ import annotations
@@ -24,6 +26,12 @@ import subprocess
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
+# a checkout of the reference project, whose sources oracle/Makefile compiles into oracle/_ref
+REFERENCE_DIR = os.environ.get("BICOS_REFERENCE_DIR", "")
+
+
+def reference_sources_present() -> bool:
+    return bool(REFERENCE_DIR) and os.path.exists(os.path.join(REFERENCE_DIR, "src", "impl", "cpu.cpp"))
 
 CV_8U, CV_16U, CV_16S, CV_32F, CV_64F = 0, 2, 3, 5, 6
 FLAG_NODUPES, FLAG_CONSISTENCY = 1, 2

@@ -17,7 +17,7 @@ def oracles():
     """The CPU checkers (test infrastructure). Builds them if needed; `ref` may be unavailable."""
     import oracle
 
-    oracle.build(ref=os.path.exists("/root/reference/src/impl/cpu.cpp"))
+    oracle.build(ref=oracle.reference_sources_present())
     return oracle
 
 

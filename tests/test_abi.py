@@ -120,9 +120,11 @@ def test_product_never_imports_the_oracle():
 
 def test_reference_pybicos_module_loads_our_library(built, tmp_path):
     """The UNMODIFIED reference pybicos/__init__.py binds our pybicos_c.so (drop-in at the FFI)."""
-    ref_init = "/root/reference/pybicos/__init__.py"
-    if not os.path.exists(ref_init):
-        pytest.skip("reference checkout not present on this machine")
+    import oracle
+
+    ref_init = os.path.join(oracle.REFERENCE_DIR, "pybicos", "__init__.py")
+    if not oracle.REFERENCE_DIR or not os.path.exists(ref_init):
+        pytest.skip("needs a checkout of the reference project (BICOS_REFERENCE_DIR)")
     pkg = tmp_path / "pybicos"
     pkg.mkdir()
     os.symlink(ref_init, pkg / "__init__.py")

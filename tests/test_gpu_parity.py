@@ -445,35 +445,59 @@ def test_randomised_configurations(handle, oracles):
     assert checked == 48
 
 
+def _reference_outputs():
+    import importlib.util
+    import os
+
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "make_reference_outputs.py")
+    spec = importlib.util.spec_from_file_location("make_reference_outputs", path)
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
 def test_match_against_unmodified_reference(handle, oracles):
-    """Same comparison, but against the compiled reference sources themselves (when they travelled)."""
-    if not oracles.ref.available():
-        pytest.skip("oracle/_ref/libbicos_ref.so not present")
-    left, right, _ = synth.make_stacks(33, 512, 400, np.uint8, seed=99, row0=256, rows=64)
-    for kw in (dict(nxcorr_threshold=0.96, min_variance=2.0),
-               dict(nxcorr_threshold=0.96, min_variance=2.0, subpixel_step=0.1, consistency=True, max_lr_diff=1)):
-        want_d, want_c = oracles.ref.match(left, right, **kw)
+    """Same comparison, but against the compiled reference sources themselves, or without them against the
+    reference's outputs stored in tests/golden/reference/ (tests/golden/make_reference_outputs.py)."""
+    ro = _reference_outputs()
+    left, right = ro.gpu_inputs()
+    live = oracles.ref.available()
+    if not live:
+        ro.check_inputs("gpu_match", left, right)
+    for i, kw in enumerate(ro.GPU_KWS):
         disp, corr = handle.match(_cuda(left), _cuda(right), Config(**kw))
-        assert _same(disp.cpu().numpy(), want_d)
-        assert _same(corr.cpu().numpy(), want_c)
+        got_d, got_c = disp.cpu().numpy(), corr.cpu().numpy()
+        if live:
+            want_d, want_c = oracles.ref.match(left, right, **kw)
+            assert _same(got_d, want_d)
+            assert _same(got_c, want_c)
+        else:
+            ro.check(f"gpu_match/{i}/disp", got_d)
+            ro.check(f"gpu_match/{i}/corr", got_c)
 
 
 def test_double_precision_against_reference_cuda_build(handle, oracles):
     """Pins the double-precision NXC (which the reference's CPU build does not have) against the
-    reference's own CUDA backend, compiled unmodified for sm_100a (oracle/_ref/libbicos_refcuda.so):
-    same valid mask, correlation within 1e-12 wherever the reference evaluated it. Integer mode:
-    the reference's CUDA build contracts the subpixel polynomial, so subpixel results are not
+    reference's own CUDA backend, compiled unmodified for sm_100a (oracle/_ref/libbicos_refcuda.so), or without
+    it against that backend's outputs stored in tests/golden/reference/ (the whole disparity, the corrmap on a
+    seeded sample of pixels): same valid mask, correlation within 1e-12 wherever the reference evaluated it.
+    Integer mode: the reference's CUDA build contracts the subpixel polynomial, so subpixel results are not
     comparable bit for bit (covered against the CPU oracle instead)."""
     import oracle
 
-    if not oracle.refcuda.available():
-        pytest.skip("oracle/_ref/libbicos_refcuda.so not present (make -C oracle refcuda)")
-    for n, dtype, kw in ((33, np.uint8, dict(nxcorr_threshold=0.9, min_variance=2.0, double=True)),
-                         (16, np.uint16, dict(nxcorr_threshold=0.9, mode_full=True, double=True, consistency=True))):
-        left, right, _ = synth.make_stacks(n, 512, 384, dtype, seed=41, row0=200, rows=64)
-        ref_d, ref_c = oracle.refcuda.match(left, right, **kw)
+    ro = _reference_outputs()
+    live = oracle.refcuda.available()
+    for n, dtype, kw in ro.DOUBLE_CASES:
+        left, right = ro.double_inputs(n, dtype)
         disp, corr = handle.match(_cuda(left), _cuda(right), Config(**kw))
         got_d, got_c = disp.cpu().numpy(), corr.cpu().numpy()
+        sample = slice(None)
+        if live:
+            ref_d, ref_c = oracle.refcuda.match(left, right, **kw)
+        else:
+            ro.check_inputs(f"double_{n}", left, right)
+            ref_d, ref_c = ro.stored()[1][f"double_{n}_disp"], ro.stored()[1][f"double_{n}_corr_sample"]
+            sample = ro.double_sample(*got_d.shape)
         assert ref_d.dtype == np.int16 and ref_c.dtype == np.float64 and got_c.dtype == np.float64
         valid_ref = ref_d != -32768
         valid_got = got_d != -32768
@@ -482,6 +506,7 @@ def test_double_precision_against_reference_cuda_build(handle, oracles):
         # the reference leaves corrmap cells it never evaluated uninitialised: compare where we evaluated
         ev = ~np.isnan(got_c)
         assert ev.sum() > 0.5 * ev.size
+        ref_c, got_c, ev = ref_c.reshape(-1), got_c.reshape(-1)[sample], ev.reshape(-1)[sample]
         assert np.max(np.abs(ref_c[ev] - got_c[ev])) <= 1e-12
 
 

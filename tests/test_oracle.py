@@ -60,56 +60,81 @@ def test_port_matches_golden(oracles, name):
         assert _same(d2, want) and _same(c2, g["corr"])
 
 
-@pytest.mark.parametrize("n,dtype,full", [(2, np.uint8, False), (3, np.uint16, True), (9, np.uint8, False),
-                                          (12, np.uint8, True), (16, np.uint16, True), (20, np.uint16, False),
-                                          (33, np.uint8, False), (65, np.uint8, False)])
+def _reference_outputs():
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("make_reference_outputs", os.path.join(GOLDEN, "make_reference_outputs.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+RO = _reference_outputs()
+
+
+@pytest.mark.parametrize("n,dtype,full", RO.BUILD_CASES)
 def test_port_matches_reference_build(oracles, n, dtype, full):
-    if not oracles.ref.available():
-        pytest.skip("reference sources not present on this machine")
-    left, right, _ = synth.make_stacks(n, 512, 150, dtype, seed=n, row0=130, rows=40)
-    assert np.array_equal(oracles.ref.descriptors(left, full), oracles.port.descriptors(left, full))
-    for kw in (dict(nxcorr_threshold=None), dict(nxcorr_threshold=0.9, min_variance=2.0),
-               dict(nxcorr_threshold=0.8, subpixel_step=0.1, consistency=True, max_lr_diff=1),
-               dict(nxcorr_threshold=0.8, subpixel_step=0.3, consistency=True, max_lr_diff=0, no_dupes=True,
-                    min_variance=0.5)):
-        a = oracles.ref.match(left, right, mode_full=full, **kw)
+    """The port against the reference build, or without it against the reference's outputs stored in
+    tests/golden/reference/ (tests/golden/make_reference_outputs.py)."""
+    live = oracles.ref.available()
+    key = f"port_build/{n}_{np.dtype(dtype).name}_{int(full)}"
+    left, right = RO.build_inputs(n, dtype)
+    desc = oracles.port.descriptors(left, full)
+    if live:
+        assert np.array_equal(oracles.ref.descriptors(left, full), desc)
+    else:
+        RO.check_inputs(key, left, right)
+        RO.check(f"{key}/desc", desc)
+    for i, kw in enumerate(RO.BUILD_KWS):
         b = oracles.port.match(left, right, mode_full=full, **kw)
-        assert _same(a[0], b[0])
-        assert (a[1] is None and b[1] is None) or _same(a[1], b[1])
+        if live:
+            a = oracles.ref.match(left, right, mode_full=full, **kw)
+            assert _same(a[0], b[0])
+            assert (a[1] is None and b[1] is None) or _same(a[1], b[1])
+        else:
+            RO.check(f"{key}/{i}/disp", b[0])
+            RO.check(f"{key}/{i}/corr", b[1])
 
 
-@pytest.mark.parametrize("n,dtype", [(17, np.uint8), (20, np.uint16), (21, np.uint16), (23, np.uint8)])
+@pytest.mark.parametrize("n,dtype", RO.WIDE_CASES)
 def test_wide_extension_matches_reference_stage_templates(oracles, n, dtype):
     """FULL stacks of 17..23 images need 258..486 bits; the reference's driver throws above 256. The port's
-    12- and 16-word paths are pinned against the reference's own stage templates with std::bitset<384/512>."""
-    if not oracles.ref.available():
-        pytest.skip("reference sources not present on this machine")
-    left, right, _ = synth.make_stacks(n, 512, 150, dtype, seed=n, row0=130, rows=16)
+    12- and 16-word paths are pinned against the reference's own stage templates with std::bitset<384/512>
+    (without the reference build: against their outputs stored in tests/golden/reference/)."""
+    live = oracles.ref.available()
+    key = f"wide/{n}_{np.dtype(dtype).name}"
+    left, right = RO.build_inputs(n, dtype, rows=16)
     k = oracles.words_per_descriptor(n, True, wide=True)
     assert k == (12 if n <= 20 else 16)
-    a, b = oracles.ref.descriptors(left, True, wide=True), oracles.port.descriptors(left, True, wide=True)
-    assert a.shape[2] == k and np.array_equal(a, b)
+    b = oracles.port.descriptors(left, True, wide=True)
+    assert b.shape[2] == k
+    if live:
+        assert np.array_equal(oracles.ref.descriptors(left, True, wide=True), b)
+    else:
+        RO.check_inputs(key, left, right)
+        RO.check(f"{key}/desc", b)
     assert (b[..., 8:] != 0).any(), "the words beyond 256 bits must be in use"
-    for kw in (dict(nxcorr_threshold=None), dict(nxcorr_threshold=0.9, min_variance=2.0),
-               dict(nxcorr_threshold=0.8, subpixel_step=0.25, consistency=True, max_lr_diff=1, no_dupes=True)):
-        x = oracles.ref.match(left, right, mode_full=True, wide_descriptors=True, **kw)
+    for i, kw in enumerate(RO.WIDE_KWS):
         y = oracles.port.match(left, right, mode_full=True, wide_descriptors=True, **kw)
-        assert _same(x[0], y[0])
-        assert (x[1] is None and y[1] is None) or _same(x[1], y[1])
+        if live:
+            x = oracles.ref.match(left, right, mode_full=True, wide_descriptors=True, **kw)
+            assert _same(x[0], y[0])
+            assert (x[1] is None and y[1] is None) or _same(x[1], y[1])
+        else:
+            RO.check(f"{key}/{i}/disp", y[0])
+            RO.check(f"{key}/{i}/corr", y[1])
     with pytest.raises(RuntimeError, match="too large"):
         oracles.port.match(left, right, mode_full=True)
 
 
 def test_search_ties_against_reference_build(oracles):
-    """Random low-entropy descriptors: many exact ties, all three flag combinations, K = 1..16."""
-    if not oracles.ref.available():
-        pytest.skip("reference sources not present on this machine")
-    rng = np.random.default_rng(0)
-    for k in (1, 2, 4, 8, 12, 16):
-        d0 = rng.integers(0, 8, size=(5, 90, k)).astype(np.uint32)
-        d1 = rng.integers(0, 8, size=(5, 90, k)).astype(np.uint32)
+    """Random low-entropy descriptors: many exact ties, all three flag combinations, K = 1..16, against the
+    reference build or without it against its results stored in tests/golden/reference/."""
+    for k, (d0, d1) in RO.tie_descriptors().items():
         for flags in (1, 2, 3):
-            assert np.array_equal(oracles.ref.bicos(d0, d1, flags, 2), oracles.port.bicos(d0, d1, flags, 2))
+            got = oracles.port.bicos(d0, d1, flags, 2)
+            want = oracles.ref.bicos(d0, d1, flags, 2) if oracles.ref.available() else RO.stored()[1][f"ties_k{k}_f{flags}"]
+            assert np.array_equal(want, got), (k, flags)
 
 
 def test_errors_follow_reference(oracles):

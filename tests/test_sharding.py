@@ -117,7 +117,7 @@ def _gpu_worker(rank, world, port, tmp):
 def test_row_sharded_match_on_two_gpus(tmp_path, oracles):
     """World size 2 over NCCL on real GPUs: peer-memory assembly and gather both equal the oracle."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     world = 2
     port = 29600 + os.getpid() % 2000
     mp.spawn(_gpu_worker, args=(world, port, str(tmp_path)), nprocs=world, join=True)
