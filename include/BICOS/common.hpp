@@ -77,6 +77,12 @@ namespace Variant {
 
 using SearchVariant = std::variant<Variant::NoDuplicates, Variant::Consistency>;
 
+// Bounds of the disparity x_left - x_right a match may have, both inclusive; min may be negative.
+struct DisparityRange {
+    int min;
+    int max;
+};
+
 struct Config {
     // Matches whose normalised cross correlation over the stack is below this are dropped.
     // Unset: no correlation stage at all, the result is the raw int16 disparity. A negative
@@ -95,6 +101,17 @@ struct Config {
     // Extension beyond the reference (leave false for its behaviour): descriptors of 384 and 512
     // bits, i.e. FULL stacks of 17..23 images, which the reference rejects as "too large".
     bool wide_descriptors = false;
+    // Extension beyond the reference (leave unset for its behaviour, the search over the whole row):
+    // search only the pairs (left column i, right column j) with min <= i - j <= max. The forward
+    // search of i runs over right columns [i - max, i - min], the reverse search of the Consistency
+    // check from right column b over left columns [b + min, b + max], both clipped to the image;
+    // ties are decided as without a range. A left pixel with no right column in range is invalid.
+    // Fewer wrong matches outside the rig's working volume, and D = max - min + 1 instead of W
+    // candidates per pixel. The range bounds the search, not the refined value: the subpixel
+    // refinement still looks at the two neighbours of the match, so a subpixel disparity may lie up
+    // to 1 px outside [min, max]. min > max throws BICOS::Exception; other values are accepted: bounds
+    // beyond +-(cols - 1) select no further pairs, and a range that covers the whole row is the same as unset.
+    std::optional<DisparityRange> disparity_range = std::nullopt;
 };
 
 // Thrown for invalid input (fewer than two images, unsupported depth, mismatching stacks) and

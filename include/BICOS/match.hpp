@@ -23,6 +23,9 @@
 // mismatching image sizes/types inside a stack throw (undefined behaviour in the reference).
 // A negative nxcorr_threshold is honoured as a threshold here (the NXC is evaluated, nothing is
 // rejected); only the Python C ABI keeps the reference's "negative = unset" (src/pybicos_c.cpp:59-69).
+// Extension: cfg.disparity_range (common.hpp) bounds the search of match and match_sharded to
+// min <= x_left - x_right <= max; left pixels without a right column in range are invalid, and
+// min > max throws BICOS::Exception.
 #pragma once
 
 #include "common.hpp"

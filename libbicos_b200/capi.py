@@ -10,7 +10,7 @@ from __future__ import annotations
 import ctypes
 import os
 from dataclasses import dataclass
-from typing import Optional, Sequence
+from typing import Optional, Sequence, Tuple
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libbicos_b200.so")
@@ -22,7 +22,7 @@ MAX_IMAGES = 65
 EXPORTS = (
     "bicos_b200_last_error", "bicos_b200_device_count", "bicos_b200_create", "bicos_b200_destroy",
     "bicos_b200_descriptor_words", "bicos_b200_disparity_type", "bicos_b200_corrmap_type",
-    "bicos_b200_transform", "bicos_b200_search", "bicos_b200_refine", "bicos_b200_match",
+    "bicos_b200_transform", "bicos_b200_search", "bicos_b200_search_range", "bicos_b200_refine", "bicos_b200_match",
     "bicos_b200_match_batch", "bicos_b200_set_overlap", "bicos_b200_match_host", "bicos_b200_match_host_begin", "bicos_b200_match_host_end", "bicos_b200_match_rows", "bicos_b200_synchronize",
     "bicos_b200_kernel_launches", "bicos_b200_set_profiling", "bicos_b200_stage_times",
     "bicos_b200_shared_alloc", "bicos_b200_shared_open", "bicos_b200_shared_close", "bicos_b200_shared_free",
@@ -50,6 +50,9 @@ class CConfig(ctypes.Structure):
         ("no_dupes", ctypes.c_int),
         ("negative_threshold_is_set", ctypes.c_int),  # extension, see include/bicos_b200.h
         ("wide_descriptors", ctypes.c_int),  # extension: 384 / 512-bit descriptors (FULL, 17..23 images)
+        ("has_disparity_range", ctypes.c_int),  # extension: search only min_disparity <= x_left - x_right <= max_disparity
+        ("min_disparity", ctypes.c_int),
+        ("max_disparity", ctypes.c_int),
     ]
 
 
@@ -66,16 +69,21 @@ class Config:
     max_lr_diff: int = 1
     no_dupes: bool = False
     wide_descriptors: bool = False  # extension beyond the reference: FULL stacks of 17..23 images
+    # extension beyond the reference: (min, max), both inclusive, of x_left - x_right; None = the whole row.
+    # See BICOS::Config::disparity_range.
+    disparity_range: Optional[Tuple[int, int]] = None
 
     def to_c(self) -> CConfig:
         def opt(v):
             return -1.0 if v is None else float(v)
 
         negative = self.nxcorr_threshold is not None and not self.nxcorr_threshold >= 0
+        rng = self.disparity_range
         return CConfig(opt(self.nxcorr_threshold), opt(self.subpixel_step), opt(self.min_variance),
                        int(self.mode_full), int(self.double), int(self.consistency),
                        int(self.max_lr_diff), int(self.no_dupes), int(negative),
-                       int(self.wide_descriptors))
+                       int(self.wide_descriptors), int(rng is not None),
+                       int(rng[0]) if rng is not None else 0, int(rng[1]) if rng is not None else 0)
 
     @property
     def flags(self) -> int:
@@ -113,6 +121,7 @@ def lib():
         L.bicos_b200_corrmap_type.argtypes = [cfgp]
         L.bicos_b200_transform.argtypes = [vp, pp, i, i, i, sz, i, i, vp, sz, vp]
         L.bicos_b200_search.argtypes = [vp, vp, vp, i, i, i, sz, i, vp, vp, vp, vp, vp]
+        L.bicos_b200_search_range.argtypes = [vp, vp, vp, i, i, i, sz, i, vp, vp, vp, vp, i, i, vp]
         L.bicos_b200_refine.argtypes = [vp, pp, pp, i, i, i, sz, i, cfgp, vp, vp, vp, vp, vp, vp, sz, vp, sz, vp]
         L.bicos_b200_match.argtypes = [vp, pp, pp, i, i, i, sz, i, cfgp, vp, sz, vp, sz, vp]
         L.bicos_b200_match_batch.argtypes = [vp, i, vp, vp, i, i, i, sz, i, cfgp, vp, sz, vp, sz, vp]
@@ -231,7 +240,7 @@ class Handle:
                                           desc.data_ptr(), pitch_words, self._stream()))
         return desc, k
 
-    def search(self, desc0, desc1, k: int, cols: int, flags: int, top_bit_free=False):
+    def search(self, desc0, desc1, k: int, cols: int, flags: int, top_bit_free=False, disparity_range=None):
         """Row-wise search on pitched descriptors -> (fwd_first, fwd_last, rev_first, rev_last).
 
         Each is a [rows, cols] int32 tensor holding uint32 keys cost << 16 | column (see
@@ -239,7 +248,8 @@ class Handle:
         vouches that bit 32k-1 of every descriptor is zero (BICOS_B200_FLAG_TOP_BIT_FREE; true for
         transform() output), which lets the tensor-core engine use its column-term kernels; ``top_bit_free=2``: the
         top TWO bits are zero (BICOS_B200_FLAG_TOP2_BITS_FREE; also true for transform() output), which adds the
-        one-pass consistency kernel."""
+        one-pass consistency kernel. ``disparity_range`` = (min, max): only the pairs with min <= x_left - x_right <= max
+        (bicos_b200_search_range); fwd_last is then always returned, and refine() needs a Config with the same range."""
         import torch
 
         rows, pitch_words = desc0.shape
@@ -249,13 +259,17 @@ class Handle:
             return torch.empty((rows, cols), dtype=torch.int32, device=dev) if needed else None
 
         fwdf = keys(True)
-        fwdl = keys(flags & FLAG_NODUPES)
+        fwdl = keys(flags & FLAG_NODUPES or disparity_range is not None)
         revf = keys(flags & FLAG_CONSISTENCY)
         revl = keys(flags == (FLAG_NODUPES | FLAG_CONSISTENCY))
         ptr = [t.data_ptr() if t is not None else None for t in (fwdf, fwdl, revf, revl)]
-        _check(lib().bicos_b200_search(self._h, desc0.data_ptr(), desc1.data_ptr(), k, rows, cols, pitch_words,
-                                       flags | (FLAG_TOP2_BITS_FREE if int(top_bit_free) >= 2 else FLAG_TOP_BIT_FREE if top_bit_free else 0),
-                                       *ptr, self._stream()))
+        flags |= FLAG_TOP2_BITS_FREE if int(top_bit_free) >= 2 else FLAG_TOP_BIT_FREE if top_bit_free else 0
+        if disparity_range is None:
+            _check(lib().bicos_b200_search(self._h, desc0.data_ptr(), desc1.data_ptr(), k, rows, cols, pitch_words, flags,
+                                           *ptr, self._stream()))
+        else:
+            _check(lib().bicos_b200_search_range(self._h, desc0.data_ptr(), desc1.data_ptr(), k, rows, cols, pitch_words, flags,
+                                                 *ptr, int(disparity_range[0]), int(disparity_range[1]), self._stream()))
         return fwdf, fwdl, revf, revl
 
     def _outputs(self, cfg: Config, rows: int, cols: int, device):

@@ -270,6 +270,24 @@ bool has_thr(const bicos_b200_config* cfg) {
     return cfg->nxcorr_threshold >= 0 || cfg->negative_threshold_is_set != 0;
 }
 
+// the configuration's disparity range clipped to the row; false when there is none or it covers the whole row,
+// which is the same search (bicos_b200_config::has_disparity_range)
+bool cfg_range(const bicos_b200_config* cfg, int cols, int* dmin, int* dmax) {
+    if (!cfg->has_disparity_range)
+        return false;
+    *dmin = cfg->min_disparity;
+    *dmax = cfg->max_disparity;
+    return disparity_range_clip(cols, dmin, dmax);
+}
+
+// the windowed search has no tensor-core kernel: a forced tensor engine fails as for its other unsupported shapes
+int check_range_engine() {
+    if (search_engine() == 2)
+        return fail(BICOS_B200_ERR_CUDA, "the tensor-core search engine has no disparity-range kernel (BICOS_B200_SEARCH_AUTO or "
+                                         "BICOS_B200_SEARCH_POPC run ranged searches)");
+    return 0;
+}
+
 size_t depth_bytes(int depth) {
     return depth == BICOS_B200_16U ? 2 : 1;
 }
@@ -334,6 +352,8 @@ int validate_common(int n, int rows, int cols, int depth, const bicos_b200_confi
         return fail(BICOS_B200_ERR_INVALID, "image too large: at most 32767 columns (int16 disparity) and 65535 rows");
     if (has_thr(cfg) && cfg->subpixel_step == 0.0f)
         return fail(BICOS_B200_ERR_INVALID, "subpixel_step must be positive (the reference loops forever on 0)");
+    if (cfg->has_disparity_range && cfg->min_disparity > cfg->max_disparity)
+        return fail(BICOS_B200_ERR_INVALID, "disparity range [%d, %d]: min > max", cfg->min_disparity, cfg->max_disparity);
     if (K_out)
         *K_out = K;
     return 0;
@@ -419,18 +439,19 @@ size_t desc_pitch_for(int cols, int K) {
     return ((size_t)cols * K + 3) & ~(size_t)3; // rows start 16 B aligned
 }
 
-int key_arrays(int flags) {
-    return 1 + ((flags & FLAG_NODUPES) ? 1 : 0) + ((flags & FLAG_CONSISTENCY) ? ((flags & FLAG_NODUPES) ? 2 : 1) : 0);
+// `ranged`: the windowed search writes fwd_last for every flags (launch_search_range)
+int key_arrays(int flags, bool ranged) {
+    return 1 + ((flags & FLAG_NODUPES) || ranged ? 1 : 0) + ((flags & FLAG_CONSISTENCY) ? ((flags & FLAG_NODUPES) ? 2 : 1) : 0);
 }
 
 struct KeyArrays {
     uint32_t *fwd_first, *fwd_last, *rev_first, *rev_last;
 };
 
-KeyArrays split_keys(uint32_t* base, size_t px, int flags) {
+KeyArrays split_keys(uint32_t* base, size_t px, int flags, bool ranged) {
     KeyArrays k { base, nullptr, nullptr, nullptr };
     uint32_t* next = base + px;
-    if (flags & FLAG_NODUPES) {
+    if ((flags & FLAG_NODUPES) || ranged) {
         k.fwd_last = next;
         next += px;
     }
@@ -489,7 +510,9 @@ int do_refine(
         prm.nsteps = h->xs_count;
         prm.xs = static_cast<const float*>(h->xs.ptr);
     }
-    prm.nodupes_forward = (search_flags(cfg) & FLAG_NODUPES) != 0;
+    int dmin = 0, dmax = 0;
+    // ranged keys: the first / last comparison also rejects the empty windows (launch_search_range)
+    prm.nodupes_forward = (search_flags(cfg) & FLAG_NODUPES) != 0 || cfg_range(cfg, cols, &dmin, &dmax);
     prm.fwd_first = fwd_first;
     prm.fwd_last = fwd_last;
     prm.rev_first = rev_first;
@@ -514,6 +537,8 @@ struct Unit {
 
 struct MatchShape {
     int n, cols, K, depth, flags;
+    bool ranged; // a disparity range that excludes some pairs: the windowed search, [dmin, dmax] clipped
+    int dmin, dmax;
     size_t pitch_bytes, disparity_pitch, corrmap_pitch;
     const bicos_b200_config* cfg;
 };
@@ -548,9 +573,17 @@ int enqueue_search_stage(bicos_b200_handle h, const Unit& u, const MatchShape& s
     }
     Range nvtx("bicos_b200::search");
     StageTimer timer(h, 1, stream);
-    KeyArrays ka = split_keys(keys, px, sh.flags);
+    KeyArrays ka = split_keys(keys, px, sh.flags, sh.ranged);
+    if (sh.ranged) {
+        if (sh.flags & FLAG_CONSISTENCY) // reverse minima merge across CTAs with atomicMin; the forward keys are stored
+            CU(cudaMemsetAsync(ka.rev_first, 0xFF, px * sizeof(uint32_t) * ((sh.flags & FLAG_NODUPES) ? 2 : 1), stream));
+        CU(launch_search_range(d0, d1, sh.K, u.nrows, sh.cols, dpw, sh.flags, sh.dmin, sh.dmax, ka.fwd_first, ka.fwd_last, ka.rev_first,
+                               ka.rev_last, stream));
+        h->launches += 1;
+        return timer.end();
+    }
     if (search_needs_prefill(sh.K, sh.cols)) // the popcount engine merges with atomicMin; the tensor-core engine stores every key
-        CU(cudaMemsetAsync(keys, 0xFF, px * sizeof(uint32_t) * key_arrays(sh.flags), stream));
+        CU(cudaMemsetAsync(keys, 0xFF, px * sizeof(uint32_t) * key_arrays(sh.flags, false), stream));
     // descriptors of our own transform: 4n - 6 or n^2 - 2n + 3 bits, never all 32 K, so the top bit is free
     CU(launch_search(d0, d1, sh.K, u.nrows, sh.cols, dpw, sh.flags, ka.fwd_first, ka.fwd_last, ka.rev_first, ka.rev_last, stream, 2)); // the transform leaves the top two descriptor bits clear
     h->launches += 1;
@@ -561,7 +594,7 @@ int enqueue_search_stage(bicos_b200_handle h, const Unit& u, const MatchShape& s
 int enqueue_refine_stage(bicos_b200_handle h, const Unit& u, const MatchShape& sh, uint32_t* keys, cudaStream_t stream) {
     Range nvtx("bicos_b200::postfilter+refine");
     StageTimer timer(h, 2, stream);
-    KeyArrays ka = split_keys(keys, (size_t)u.nrows * sh.cols, sh.flags);
+    KeyArrays ka = split_keys(keys, (size_t)u.nrows * sh.cols, sh.flags, sh.ranged);
     if (int rc = do_refine(h, u.t0, u.t1, sh.n, u.nrows, sh.cols, sh.pitch_bytes, sh.depth, sh.cfg, ka.fwd_first, ka.fwd_last, ka.rev_first,
                            ka.rev_last, nullptr, u.disp_rows, sh.disparity_pitch, u.corr_rows, sh.corrmap_pitch, stream))
         return rc;
@@ -582,6 +615,10 @@ int validate_match(const void* const* planes0, const void* const* planes1, int n
     sh.K = K;
     sh.depth = depth;
     sh.flags = search_flags(cfg);
+    sh.ranged = cfg_range(cfg, cols, &sh.dmin, &sh.dmax);
+    if (sh.ranged)
+        if (int rc = check_range_engine())
+            return rc;
     sh.pitch_bytes = pitch_bytes;
     sh.cfg = cfg;
     return 0;
@@ -593,7 +630,7 @@ int reserve_workspace(bicos_b200_handle h, const MatchShape& sh, int max_unit_ro
     CU(h->desc1.reserve(dpw * max_unit_rows * sizeof(uint32_t)));
     // key arrays, contiguous so that one memset initialises them: fwd_first, then fwd_last
     // (NODUPES), rev_first (CONSISTENCY), rev_last (both)
-    const size_t key_bytes = (size_t)max_unit_rows * sh.cols * sizeof(uint32_t) * key_arrays(sh.flags);
+    const size_t key_bytes = (size_t)max_unit_rows * sh.cols * sizeof(uint32_t) * key_arrays(sh.flags, sh.ranged);
     CU(h->keys.reserve(key_bytes));
     if (second_keys)
         CU(h->keys_b.reserve(key_bytes));
@@ -865,6 +902,43 @@ int bicos_b200_search(bicos_b200_handle h, const uint32_t* desc0, const uint32_t
     return 0;
 }
 
+int bicos_b200_search_range(bicos_b200_handle h, const uint32_t* desc0, const uint32_t* desc1, int K, int rows, int cols,
+                            size_t desc_pitch_words, int flags, uint32_t* fwd_first, uint32_t* fwd_last, uint32_t* rev_first,
+                            uint32_t* rev_last, int min_disparity, int max_disparity, void* stream) {
+    if (min_disparity > max_disparity)
+        return fail(BICOS_B200_ERR_INVALID, "disparity range [%d, %d]: min > max", min_disparity, max_disparity);
+    if (cols <= 0 || !disparity_range_clip(cols, &min_disparity, &max_disparity))
+        return bicos_b200_search(h, desc0, desc1, K, rows, cols, desc_pitch_words, flags, fwd_first, fwd_last, rev_first, rev_last,
+                                 stream);
+    if (!h || !desc0 || !desc1 || !fwd_first || !fwd_last)
+        return fail(BICOS_B200_ERR_INVALID, "null argument (a ranged search always needs fwd_last)");
+    if (K != 1 && K != 2 && K != 4 && K != 8 && K != 12 && K != 16)
+        return fail(BICOS_B200_ERR_INVALID, "K must be 1, 2, 4 or 8 (12 or 16 for wide descriptors)");
+    if (flags < 0 || flags > 15)
+        return fail(BICOS_B200_ERR_INVALID, "bad flags");
+    flags &= 3; // the top-bit promises only matter to the tensor-core engine
+    if (rows <= 0 || rows > 65535 || cols > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "bad image size");
+    if ((flags & FLAG_CONSISTENCY) && (!rev_first || ((flags & FLAG_NODUPES) && !rev_last)))
+        return fail(BICOS_B200_ERR_INVALID, "consistency search needs rev_first (and rev_last with no_dupes)");
+    if (desc_pitch_words < (size_t)cols * K || (desc_pitch_words % 4) != 0)
+        return fail(BICOS_B200_ERR_INVALID, "descriptor rows must be 16-byte aligned and hold cols*K words");
+    if (int rc = check_range_engine())
+        return rc;
+    DeviceGuard g(h->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const size_t bytes = (size_t)rows * cols * sizeof(uint32_t);
+    if (flags & FLAG_CONSISTENCY) {
+        CU(cudaMemsetAsync(rev_first, 0xFF, bytes, s));
+        if (flags & FLAG_NODUPES)
+            CU(cudaMemsetAsync(rev_last, 0xFF, bytes, s));
+    }
+    CU(launch_search_range(desc0, desc1, K, rows, cols, desc_pitch_words, flags, min_disparity, max_disparity, fwd_first, fwd_last,
+                           rev_first, rev_last, s));
+    h->launches += 1;
+    return 0;
+}
+
 int bicos_b200_refine(bicos_b200_handle h, const void* const* planes0, const void* const* planes1,
                       int n, int rows, int cols, size_t pitch_bytes, int depth,
                       const bicos_b200_config* cfg, const uint32_t* fwd_first, const uint32_t* fwd_last,
@@ -875,8 +949,11 @@ int bicos_b200_refine(bicos_b200_handle h, const void* const* planes0, const voi
         return fail(BICOS_B200_ERR_INVALID, "null argument");
     if (int rc = validate_common(n, rows, cols, depth, cfg, nullptr))
         return rc;
+    int dmin = 0, dmax = 0;
     if ((search_flags(cfg) & FLAG_NODUPES) && !fwd_last)
         return fail(BICOS_B200_ERR_INVALID, "no-duplicates postfilter needs fwd_last");
+    if (cfg_range(cfg, cols, &dmin, &dmax) && !fwd_last)
+        return fail(BICOS_B200_ERR_INVALID, "a ranged postfilter needs fwd_last (bicos_b200_search_range)");
     if (cfg->variant_type != 0 && (!rev_first || (cfg->no_dupes && !rev_last)))
         return fail(BICOS_B200_ERR_INVALID, "consistency postfilter needs rev_first (and rev_last with no_dupes)");
     DeviceGuard g(h->device);
@@ -894,7 +971,7 @@ int bicos_b200_refine(bicos_b200_handle h, const void* const* planes0, const voi
 // pipeline, band b + 1's search beside band b's refine. Rows are independent, so the result is the same. Measured with
 // tools/overlap_probe.py --frames 1: 1536 rows 2.01 ms as one unit, 1.93 / 1.91 / 1.91 ms as 2 / 3 / 4 bands; 768 rows
 // (a shard of a two-GPU match) 1.025 -> 0.991 / 0.989 ms as 2 / 3 bands; 384 rows: no gain. Small images, integer
-// refinement and the popcount engine (which leaves no issue slots free) run as one unit.
+// refinement, the popcount engine (which leaves no issue slots free) and ranged matches run as one unit.
 static int match_banded_or_whole(bicos_b200_handle h, const void* const* planes0, const void* const* planes1, int n, int rows,
                                  int cols, size_t pitch_bytes, int depth, const bicos_b200_config* cfg, void* disparity,
                                  size_t disparity_pitch, void* corrmap, size_t corrmap_pitch, cudaStream_t stream) {
@@ -907,7 +984,8 @@ static int match_banded_or_whole(bicos_b200_handle h, const void* const* planes0
     // the one-pass consistency search takes its SM's whole register file: nothing runs beside it, and bands would only add
     // launches (1.71 against 1.63 ms on the metric configuration)
     const bool onepass = search_engine() != 1 && search_mma_supports(sh.K, cols) && search_mma_onepass_applies(sh.K, cols, sh.flags, 2);
-    if (!h->overlap || !subpixel || onepass || rows < BANDS * MIN_BAND_ROWS || search_needs_prefill(sh.K, cols) || (sh.K != 4 && sh.K != 8))
+    if (!h->overlap || !subpixel || onepass || sh.ranged || rows < BANDS * MIN_BAND_ROWS || search_needs_prefill(sh.K, cols) ||
+        (sh.K != 4 && sh.K != 8))
         return do_match(h, planes0, planes1, n, rows, cols, pitch_bytes, depth, cfg, 0, rows, disparity, disparity_pitch, corrmap,
                         corrmap_pitch, stream);
     sh.disparity_pitch = disparity_pitch;

@@ -5,6 +5,7 @@
 //
 //   bicos-cli folder0 [folder1] [-t thr] [-v var] [-s step] [-o out.png] [-n N] [-q Q.yaml]
 //             [--allow-negative-z] [-m lr-maxdiff] [--double] [--limited] [--corrmap] [--no-dupes] [--wide-descriptors]
+//             [--disparity-range MIN:MAX]
 //
 // Differences, on purpose: --allow-negative-z is honoured (the reference reads a non-existent
 // "allow-behind" option, cli.cpp:231); integer-mode disparities with a threshold are float32
@@ -61,6 +62,7 @@ const Option OPTIONS[] = {
     { "corrmap", 0, false, "Output map of normalized cross correlation values." },
     { "no-dupes", 0, false, "Default BICOS variant when --lr-maxdiff is not specified. Can be set together with --lr-maxdiff to activate both." },
     { "wide-descriptors", 0, false, "Extension: accept 17..23 images without --limited (384 / 512-bit descriptors; the reference stops at 16)." },
+    { "disparity-range", 0, true, "Extension: search only disparities MIN..MAX (inclusive, may be negative), e.g. 0:127. (default: the whole row)" },
     { "help", 'h', false, "Display this message." },
 };
 
@@ -342,6 +344,23 @@ int run(int argc, char const* const* argv) {
         c.precision = Precision::DOUBLE;
     if (args.has("wide-descriptors"))
         c.wide_descriptors = true;
+    if (args.has("disparity-range")) {
+        const std::string& v = args.get("disparity-range");
+        const size_t colon = v.find(':', 1); // a leading '-' is the sign of MIN
+        size_t used0 = 0, used1 = 0;
+        int lo = 0, hi = 0;
+        try {
+            if (colon == std::string::npos)
+                throw std::invalid_argument("no colon");
+            lo = std::stoi(v.substr(0, colon), &used0);
+            hi = std::stoi(v.substr(colon + 1), &used1);
+        } catch (const std::exception&) {
+            used0 = 0;
+        }
+        if (used0 == 0 || used0 != colon || used1 != v.size() - colon - 1)
+            throw std::invalid_argument("Option 'disparity-range' expects MIN:MAX, got '" + v + "'");
+        c.disparity_range = DisparityRange { lo, hi };
+    }
     if (args.has("lr-maxdiff"))
         c.variant = Variant::Consistency { (int)to_uint(args, "lr-maxdiff"), args.has("no-dupes") };
 

@@ -147,6 +147,38 @@ void note_search_kernel(const char* fmt, ...);
 // longer than BICOS_B200_MMA_TIMEOUT_MS, default 10 s): its keys are garbage. Clears the flag.
 unsigned int search_mma_take_timeout();
 
+// kernel 2, windowed (search_range.cu): the same search over the pairs (left i, right j) with
+// dmin <= i - j <= dmax only (Config::disparity_range; the range is clipped to [-cols, cols] here,
+// which selects the same pairs). Integer pipes, K = 1/2/4/8/12/16, rows of up to 32767 pixels, the key format of
+// launch_search. rev_first / rev_last (in use with FLAG_CONSISTENCY) must be pre-filled with
+// KEY_NONE by the caller; fwd_first and fwd_last are stored for every pixel.
+// Contract with the refine, which cannot tell that a window was empty (a left pixel with
+// i - dmin < 0 or i - dmax > cols - 1): fwd_last is ALWAYS written and required, with FLAG_NODUPES
+// as the real last-minimum key, otherwise as the mirror cost << 16 | (65535 - best) of fwd_first;
+// an empty window gets KEY_NONE in both. The refine must therefore run with nodupes_forward = 1 on
+// these keys: its first / last comparison rejects exactly the empty windows before it reads anything
+// else (rev_first of column 65535 in particular).
+cudaError_t launch_search_range(
+    const uint32_t* desc0,
+    const uint32_t* desc1,
+    int K,
+    int rows,
+    int cols,
+    size_t desc_pitch_words,
+    int flags,
+    int dmin,
+    int dmax,
+    uint32_t* fwd_first,
+    uint32_t* fwd_last,
+    uint32_t* rev_first,
+    uint32_t* rev_last,
+    cudaStream_t stream
+);
+// Clips [*dmin, *dmax] to [-cols, cols] in place (i - j lies in [-(cols-1), cols-1], so the pairs stay the
+// same); false when the range covers every pair of the row, i.e. means exactly "no range" and the full-row
+// search applies.
+bool disparity_range_clip(int cols, int* dmin, int* dmax);
+
 // kernel 3: postfilter (no-duplicates / left-right consistency) fused with the NXC
 // agree / agree_subpixel refinement (reference a7 tail, a8, a9, a10, a11)
 cudaError_t launch_refine(

@@ -61,6 +61,11 @@ bicos_b200_config to_c_config(const Config& cfg) {
     c.mode = cfg.mode == TransformMode::FULL ? 1 : 0;
     c.precision = cfg.precision == Precision::DOUBLE ? 1 : 0;
     c.wide_descriptors = cfg.wide_descriptors ? 1 : 0;
+    if (cfg.disparity_range) {
+        c.has_disparity_range = 1;
+        c.min_disparity = cfg.disparity_range->min;
+        c.max_disparity = cfg.disparity_range->max;
+    }
     if (std::holds_alternative<Variant::Consistency>(cfg.variant)) {
         const auto& v = std::get<Variant::Consistency>(cfg.variant);
         c.variant_type = 1;
