@@ -174,6 +174,52 @@ int bicos_b200_match(bicos_b200_handle h, const void* const* planes0, const void
                      const bicos_b200_config* cfg, void* disparity, size_t disparity_pitch_bytes,
                      void* corrmap, size_t corrmap_pitch_bytes, void* stream);
 
+/* ---- rectification: raw camera stacks in ------------------------------------------------
+ * The match expects rectified stacks (corresponding points on the same row). These entry points APPLY
+ * rectification maps the caller already has, e.g. from OpenCV's cv::initUndistortRectifyMap with
+ * m1type = CV_32FC1 (computing the maps from a calibration is a one-off host step and not part of this
+ * library). Semantics, bit for bit those of OpenCV's CPU cv::remap(src, dst, map_x, map_y, INTER_LINEAR,
+ * BORDER_CONSTANT, 0) on float32 maps:
+ *   X = round_half_even(map_x(y, x) * 32), Y = likewise; x0 = X >> 5, y0 = Y >> 5 (floor), fx = X & 31, fy = Y & 31
+ *   taps v00 = src(y0, x0), v01 = src(y0, x0 + 1), v10 = src(y0 + 1, x0), v11 = src(y0 + 1, x0 + 1); a tap
+ *   outside the source reads 0
+ *   8U:  dst = ((32-fx)(32-fy) v00 + fx(32-fy) v01 + (32-fx)fy v10 + fx fy v11 + 512) >> 10 (int32)
+ *   16U: float32 weights w00 = (1-ay)(1-ax), w01 = (1-ay)ax, w10 = ay(1-ax), w11 = ay ax with ax = fx/32,
+ *        ay = fy/32; dst = saturate_u16(round_half_even(((v00 w00 + v01 w01) + v10 w10) + v11 w11)), each
+ *        product and sum rounded to float32 on its own
+ *   a map value that is NaN, +-inf or of magnitude >= 2^25 gives 0
+ * The output has the maps' size (rows x cols); the source size is independent. Both are at most 32767 x 32767.
+ * Identity maps (map_x = x, map_y = y) reproduce the input exactly. */
+
+/* Stage entry point: remaps n (1..65) device planes src_planes[i] [src_rows][src_pitch_bytes] through one map
+ * pair (device float32 [rows][map_pitch_bytes], pitch a multiple of 4 and at least cols * 4) into
+ * dst_planes[i] [rows][dst_pitch_bytes]. Writes exactly the rows * cols output pixels of each plane. */
+int bicos_b200_remap(bicos_b200_handle h, const void* const* src_planes, int n, int src_rows, int src_cols,
+                     size_t src_pitch_bytes, int depth, const float* map_x, const float* map_y, size_t map_pitch_bytes,
+                     int rows, int cols, void* const* dst_planes, size_t dst_pitch_bytes, void* stream);
+
+/* The map pairs of both cameras: device float32 [rows][map_pitch_bytes] each, one pitch for all four. */
+typedef struct {
+    const float* map_x0;
+    const float* map_y0;
+    const float* map_x1;
+    const float* map_y1;
+    size_t map_pitch_bytes;
+} bicos_b200_rectify_maps;
+
+/* bicos_b200_match on raw stacks: remaps planes0 through (map_x0, map_y0) and planes1 through (map_x1, map_y1)
+ * (one launch for both) into a workspace the handle owns, then runs bicos_b200_match on the rectified
+ * [rows][cols] stacks. The result is bit-identical to bicos_b200_remap of both stacks followed by
+ * bicos_b200_match (row bands, overlap, engine choice and disparity range as for that match). The outputs
+ * have the rectified size. The workspace grows on demand (128-byte aligned rows) and lives until
+ * bicos_b200_destroy; like the rest of the handle's workspace it serves one match at a time, and a
+ * rectified match enqueued on another stream than the handle's previous match first waits for that one. */
+int bicos_b200_match_rectified(bicos_b200_handle h, const void* const* planes0, const void* const* planes1, int n,
+                               int src_rows, int src_cols, size_t src_pitch_bytes, int depth,
+                               const bicos_b200_rectify_maps* maps, int rows, int cols, const bicos_b200_config* cfg,
+                               void* disparity, size_t disparity_pitch_bytes, void* corrmap, size_t corrmap_pitch_bytes,
+                               void* stream);
+
 /* Throughput mode: `count` independent stereo stacks of one shape, type and configuration (BASELINE.json's batch
  * configuration). planes0[f] / planes1[f] are the n plane pointers of frame f, disparity[f] / corrmap[f] its outputs
  * (corrmap may be NULL, or hold NULL entries). Same results as `count` calls of bicos_b200_match, but the frames

@@ -13,8 +13,8 @@ The product path is CUDA only. Importing this package does not load the shared l
 the first call does, and fails loudly if it has not been built.
 """
 
-from .capi import (BicosError, Config, Handle, SharedImage, descriptor_words, last_search_kernel, lib,  # noqa: F401
-                   search_engine, set_search_engine)
+from .capi import (BicosError, Config, Handle, RectifyMaps, SharedImage, descriptor_words, last_search_kernel,  # noqa: F401
+                   lib, search_engine, set_search_engine)
 
-__all__ = ["BicosError", "Config", "Handle", "SharedImage", "descriptor_words", "last_search_kernel", "lib", "search_engine",
-           "set_search_engine"]
+__all__ = ["BicosError", "Config", "Handle", "RectifyMaps", "SharedImage", "descriptor_words", "last_search_kernel", "lib",
+           "search_engine", "set_search_engine"]

@@ -27,6 +27,7 @@ EXPORTS = (
     "bicos_b200_kernel_launches", "bicos_b200_set_profiling", "bicos_b200_stage_times",
     "bicos_b200_shared_alloc", "bicos_b200_shared_open", "bicos_b200_shared_close", "bicos_b200_shared_free",
     "bicos_b200_set_search_engine", "bicos_b200_get_search_engine", "bicos_b200_last_search_kernel",
+    "bicos_b200_remap", "bicos_b200_match_rectified",
 )
 SEARCH_ENGINES = {"auto": 0, "popc": 1, "tensor": 2}
 IPC_HANDLE_BYTES = 64
@@ -92,6 +93,25 @@ class Config:
         return FLAG_NODUPES
 
 
+class CRectifyMaps(ctypes.Structure):
+    """bicos_b200_rectify_maps."""
+
+    _fields_ = [("map_x0", ctypes.c_void_p), ("map_y0", ctypes.c_void_p), ("map_x1", ctypes.c_void_p),
+                ("map_y1", ctypes.c_void_p), ("map_pitch_bytes", ctypes.c_size_t)]
+
+
+@dataclass
+class RectifyMaps:
+    """Rectification maps of both cameras for Handle.match_rectified: float32 CUDA tensors [rows, cols] with
+    contiguous rows, all of one shape and row stride, e.g. the CV_32FC1 maps of cv2.initUndistortRectifyMap.
+    map_x0 / map_y0 rectify stack0, map_x1 / map_y1 stack1."""
+
+    map_x0: object
+    map_y0: object
+    map_x1: object
+    map_y1: object
+
+
 _lib = None
 
 
@@ -136,6 +156,9 @@ def lib():
         L.bicos_b200_shared_free.argtypes = [i, vp]
         L.bicos_b200_synchronize.argtypes = [vp, vp]
         L.bicos_b200_set_profiling.argtypes = [vp, i]
+        L.bicos_b200_remap.argtypes = [vp, pp, i, i, i, sz, i, vp, vp, sz, i, i, pp, sz, vp]
+        L.bicos_b200_match_rectified.argtypes = [vp, pp, pp, i, i, i, sz, i, ctypes.POINTER(CRectifyMaps), i, i, cfgp, vp, sz, vp,
+                                                 sz, vp]
         L.bicos_b200_stage_times.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_longlong)]
         _lib = L
     return _lib
@@ -372,6 +395,61 @@ class Handle:
         else:
             _check(lib().bicos_b200_match_rows(self._h, p0, p1, n, rows, cols, pitch, depth, ctypes.byref(ccfg),
                                                int(rows_range[0]), int(rows_range[1]), *args))
+        return disp, corr
+
+    @staticmethod
+    def _map_info(maps, device):
+        """(pointers, rows, cols, pitch in bytes) of float32 map tensors of one shape and row stride."""
+        import torch
+
+        first = maps[0]
+        for m in maps:
+            if not isinstance(m, torch.Tensor) or m.dtype != torch.float32 or m.dim() != 2 or not m.is_cuda:
+                raise BicosError("rectification maps must be float32 CUDA tensors of shape [rows, cols]")
+            if m.device != device:
+                raise BicosError(f"a rectification map lives on {m.device}, the stacks on {device}")
+            if m.shape != first.shape or m.stride() != first.stride() or m.stride(1) != 1:
+                raise BicosError("rectification maps must share one shape and row stride, with contiguous rows")
+        rows, cols = first.shape
+        return [m.data_ptr() for m in maps], rows, cols, first.stride(0) * 4
+
+    def remap(self, stack, map_x, map_y, out=None):
+        """Rectification stage (bicos_b200_remap): [n, src_rows, src_cols] uint8 / uint16 CUDA tensor -> [n, rows, cols] of
+        its dtype, out[i] = cv2.remap(stack[i], map_x, map_y, INTER_LINEAR, BORDER_CONSTANT, 0) bit for bit. ``map_x`` /
+        ``map_y``: float32 CUDA tensors [rows, cols]. ``out``: a tensor of that shape and dtype, contiguous rows."""
+        import torch
+
+        planes, n, src_rows, src_cols, pitch, depth = self._stack_info(stack)
+        (px, py), rows, cols, map_pitch = self._map_info([map_x, map_y], stack.device)
+        if out is None:
+            out = torch.empty((n, rows, cols), dtype=stack.dtype, device=stack.device)
+        elif (not isinstance(out, torch.Tensor) or out.dtype != stack.dtype or tuple(out.shape) != (n, rows, cols)
+              or out.device != stack.device):
+            raise BicosError(f"out must be a {stack.dtype} tensor of shape ({n}, {rows}, {cols}) on {stack.device}")
+        dst, _, _, _, dst_pitch, _ = self._stack_info(out)
+        _check(lib().bicos_b200_remap(self._h, planes, n, src_rows, src_cols, pitch, depth, px, py, map_pitch, rows, cols,
+                                      dst, dst_pitch, self._stream()))
+        return out
+
+    def match_rectified(self, stack0, stack1, maps: RectifyMaps, cfg: Config, out=None):
+        """match() on raw stacks (bicos_b200_match_rectified): both stacks are remapped through ``maps`` into the
+        handle's workspace (one launch), then matched; bit-identical to match(remap(stack0, ...), remap(stack1, ...)).
+        The outputs have the maps' shape; ``out`` = (disparity, corrmap) tensors of that shape to reuse."""
+        p0, n, src_rows, src_cols, pitch, depth = self._stack_info(stack0)
+        p1, n1, rows1, cols1, pitch1, depth1 = self._stack_info(stack1)
+        if (n1, rows1, cols1, pitch1, depth1) != (n, src_rows, src_cols, pitch, depth):
+            raise BicosError("stack0 and stack1 differ")
+        ptrs, rows, cols, map_pitch = self._map_info([maps.map_x0, maps.map_y0, maps.map_x1, maps.map_y1], stack0.device)
+        if out is None:
+            ccfg, disp, corr = self._outputs(cfg, rows, cols, stack0.device)
+        else:
+            ccfg = cfg.to_c()
+            disp, corr = self._check_out(ccfg, out, rows, cols, stack0.device)
+        cmaps = CRectifyMaps(*ptrs, map_pitch)
+        _check(lib().bicos_b200_match_rectified(
+            self._h, p0, p1, n, src_rows, src_cols, pitch, depth, ctypes.byref(cmaps), rows, cols, ctypes.byref(ccfg),
+            disp.data_ptr(), disp.stride(0) * disp.element_size(), corr.data_ptr() if corr is not None else None,
+            corr.stride(0) * corr.element_size() if corr is not None else 0, self._stream()))
         return disp, corr
 
     def match_batch(self, frames, cfg: Config, outs=None):

@@ -302,6 +302,7 @@ struct bicos_b200_handle_s {
     int device = 0;
     DeviceBuffer desc0, desc1, keys, xs; // keys: up to four [rows][cols] uint32 search-key arrays
     DeviceBuffer stage_in, stage_disp, stage_corr;
+    DeviceBuffer rect; // bicos_b200_match_rectified: both rectified stacks, [2n][rows][rect pitch]
     float xs_step = -1.f;
     int xs_count = 0;
     bool host_pending = false; // between bicos_b200_match_host_begin and _end
@@ -789,7 +790,7 @@ int bicos_b200_destroy(bicos_b200_handle h) {
     {
         DeviceGuard g(h->device);
         cudaDeviceSynchronize();
-        for (DeviceBuffer* b: { &h->desc0, &h->desc1, &h->keys, &h->xs, &h->stage_in, &h->stage_disp, &h->stage_corr })
+        for (DeviceBuffer* b: { &h->desc0, &h->desc1, &h->keys, &h->xs, &h->stage_in, &h->stage_disp, &h->stage_corr, &h->rect })
             b->release();
         for (cudaEvent_t e: h->prof_events)
             cudaEventDestroy(e);
@@ -1011,6 +1012,114 @@ int bicos_b200_match(bicos_b200_handle h, const void* const* planes0, const void
     DeviceGuard g(h->device);
     return match_banded_or_whole(h, planes0, planes1, n, rows, cols, pitch_bytes, depth, cfg, disparity,
                                  disparity_pitch_bytes, corrmap, corrmap_pitch_bytes, static_cast<cudaStream_t>(stream));
+}
+
+// checks shared by bicos_b200_remap and bicos_b200_match_rectified
+static int validate_remap(int n, int src_rows, int src_cols, size_t src_pitch_bytes, int depth, const float* map_x,
+                          const float* map_y, size_t map_pitch_bytes, int rows, int cols) {
+    if (depth != BICOS_B200_8U && depth != BICOS_B200_16U)
+        return fail(BICOS_B200_ERR_INVALID, "bad input depths, only CV_8UC1 and CV_16UC1 are supported");
+    if (n < 1 || n > MAX_IMAGES)
+        return fail(BICOS_B200_ERR_INVALID, "remap of %d planes: 1 to %d are supported", n, MAX_IMAGES);
+    if (!map_x || !map_y)
+        return fail(BICOS_B200_ERR_INVALID, "rectification map is null");
+    if (src_rows <= 0 || src_cols <= 0 || rows <= 0 || cols <= 0)
+        return fail(BICOS_B200_ERR_INVALID, "empty images");
+    if (src_rows > 32767 || src_cols > 32767 || rows > 32767 || cols > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "image too large: remap source and output have at most 32767 rows and columns");
+    if (src_pitch_bytes < (size_t)src_cols * depth_bytes(depth))
+        return fail(BICOS_B200_ERR_INVALID, "source pitch smaller than a row");
+    if (map_pitch_bytes < (size_t)cols * sizeof(float) || map_pitch_bytes % sizeof(float) != 0 ||
+        reinterpret_cast<uintptr_t>(map_x) % sizeof(float) != 0 || reinterpret_cast<uintptr_t>(map_y) % sizeof(float) != 0)
+        return fail(BICOS_B200_ERR_INVALID, "map rows must be 4-byte aligned and hold cols float32 values");
+    return 0;
+}
+
+int bicos_b200_remap(bicos_b200_handle h, const void* const* src_planes, int n, int src_rows, int src_cols,
+                     size_t src_pitch_bytes, int depth, const float* map_x, const float* map_y, size_t map_pitch_bytes,
+                     int rows, int cols, void* const* dst_planes, size_t dst_pitch_bytes, void* stream) {
+    if (!h || !src_planes || !dst_planes)
+        return fail(BICOS_B200_ERR_INVALID, "null argument");
+    if (int rc = validate_remap(n, src_rows, src_cols, src_pitch_bytes, depth, map_x, map_y, map_pitch_bytes, rows, cols))
+        return rc;
+    if (dst_pitch_bytes < (size_t)cols * depth_bytes(depth))
+        return fail(BICOS_B200_ERR_INVALID, "output pitch smaller than a row");
+    DeviceGuard g(h->device);
+    RemapParams prm {};
+    if (int rc = fill_table(prm.side[0].src, src_planes, n, 0))
+        return rc;
+    if (int rc = fill_table(prm.side[0].dst, dst_planes, n, 0))
+        return rc;
+    prm.side[0].map_x = map_x;
+    prm.side[0].map_y = map_y;
+    prm.n = n;
+    prm.src_rows = src_rows;
+    prm.src_cols = src_cols;
+    prm.rows = rows;
+    prm.cols = cols;
+    prm.src_pitch = src_pitch_bytes;
+    prm.map_pitch = map_pitch_bytes;
+    prm.dst_pitch = dst_pitch_bytes;
+    CU(launch_remap(prm, 1, depth == BICOS_B200_16U, static_cast<cudaStream_t>(stream)));
+    h->launches += 1;
+    return 0;
+}
+
+int bicos_b200_match_rectified(bicos_b200_handle h, const void* const* planes0, const void* const* planes1, int n,
+                               int src_rows, int src_cols, size_t src_pitch_bytes, int depth,
+                               const bicos_b200_rectify_maps* maps, int rows, int cols, const bicos_b200_config* cfg,
+                               void* disparity, size_t disparity_pitch_bytes, void* corrmap, size_t corrmap_pitch_bytes,
+                               void* stream) {
+    if (!h)
+        return fail(BICOS_B200_ERR_INVALID, "null handle");
+    if (!maps)
+        return fail(BICOS_B200_ERR_INVALID, "rectification maps are null");
+    const size_t pitch = ((size_t)cols * depth_bytes(depth) + 127) & ~(size_t)127; // rectified planes in the workspace
+    // everything the match would reject at the rectified size is rejected before the remap is enqueued
+    MatchShape sh {};
+    if (int rc = validate_match(planes0, planes1, n, rows, cols, pitch, depth, cfg, disparity, sh))
+        return rc;
+    for (int side = 0; side < 2; ++side)
+        if (int rc = validate_remap(n, src_rows, src_cols, src_pitch_bytes, depth, side ? maps->map_x1 : maps->map_x0,
+                                    side ? maps->map_y1 : maps->map_y0, maps->map_pitch_bytes, rows, cols))
+            return rc;
+    DeviceGuard g(h->device);
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    RemapParams prm {};
+    if (int rc = fill_table(prm.side[0].src, planes0, n, 0))
+        return rc;
+    if (int rc = fill_table(prm.side[1].src, planes1, n, 0))
+        return rc;
+    if (int rc = enter_workspace(h, s)) // the previous match of the handle may still read the rectified planes
+        return rc;
+    const size_t plane_bytes = pitch * (size_t)rows;
+    CU(h->rect.reserve(plane_bytes * 2 * (size_t)n));
+    std::vector<const void*> rect0((size_t)n), rect1((size_t)n);
+    for (int i = 0; i < n; ++i) {
+        rect0[(size_t)i] = static_cast<char*>(h->rect.ptr) + plane_bytes * (size_t)i;
+        rect1[(size_t)i] = static_cast<char*>(h->rect.ptr) + plane_bytes * (size_t)(n + i);
+    }
+    fill_table(prm.side[0].dst, rect0.data(), n, 0);
+    fill_table(prm.side[1].dst, rect1.data(), n, 0);
+    prm.side[0].map_x = maps->map_x0;
+    prm.side[0].map_y = maps->map_y0;
+    prm.side[1].map_x = maps->map_x1;
+    prm.side[1].map_y = maps->map_y1;
+    prm.n = n;
+    prm.src_rows = src_rows;
+    prm.src_cols = src_cols;
+    prm.rows = rows;
+    prm.cols = cols;
+    prm.src_pitch = src_pitch_bytes;
+    prm.map_pitch = maps->map_pitch_bytes;
+    prm.dst_pitch = pitch;
+    {
+        Range nvtx("bicos_b200::remap x2");
+        CU(launch_remap(prm, 2, depth == BICOS_B200_16U, s));
+        h->launches += 1;
+    }
+    return match_banded_or_whole(h, rect0.data(), rect1.data(), n, rows, cols, pitch, depth, cfg, disparity, disparity_pitch_bytes,
+                                 corrmap, corrmap_pitch_bytes, s);
 }
 
 int bicos_b200_match_rows(bicos_b200_handle h, const void* const* planes0,

@@ -190,4 +190,23 @@ cudaError_t launch_refine(
 
 int search_smem_bytes(int K, int cols, int flags);
 
+// stage 0 (remap.cu): rectification of n planes per side through one map pair per side, with the semantics of
+// cv::remap(INTER_LINEAR, BORDER_CONSTANT 0) on float32 maps (bicos_b200_remap). Output [rows][cols], source
+// [src_rows][src_cols], both at most 32767; maps are float32 [rows][map_pitch bytes].
+struct RemapSide {
+    PlaneTable src;
+    PlaneTable dst; // written, despite PlaneTable's const
+    const float* map_x;
+    const float* map_y;
+};
+
+struct RemapParams {
+    RemapSide side[2];
+    int n, src_rows, src_cols, rows, cols;
+    size_t src_pitch, map_pitch, dst_pitch; // bytes
+};
+
+// `sides` = 1 or 2: blockIdx.z picks prm.side[z], so both stacks of a match are one launch
+cudaError_t launch_remap(const RemapParams& prm, int sides, int is_u16, cudaStream_t stream);
+
 } // namespace bicos_b200

@@ -3,6 +3,7 @@
 // drivers (src/lib.cpp:31-49, src/impl/cpu.cpp:100-159, src/impl/cuda.cu:465-524).
 
 #include "../../include/BICOS/match.hpp"
+#include "../../include/BICOS/rectify.hpp"
 #include "../../include/bicos_b200.h"
 
 #include <cuda_runtime.h>
@@ -112,6 +113,27 @@ int device_of(const void* ptr) {
         throw Exception("input images must live in device memory");
     return attr.device;
 }
+
+// checks a map pair of the rectified size: CV_32FC1 device images of one size and pitch
+void check_maps(const Image& map_x, const Image& map_y, const Image& like) {
+    for (const Image* m: { &map_x, &map_y })
+        if (m->empty() || m->type() != IMG_32F || m->rows != like.rows || m->cols != like.cols || m->step != like.step)
+            throw Exception("rectification maps must be non-empty CV_32FC1 images of one size and pitch");
+}
+
+// makes `device` current for the scope's lifetime
+struct DeviceScope {
+    int prev = 0, device = 0;
+    explicit DeviceScope(int dev): device(dev) {
+        cuda_check(cudaGetDevice(&prev), "cudaGetDevice");
+        if (prev != device)
+            cuda_check(cudaSetDevice(device), "cudaSetDevice");
+    }
+    ~DeviceScope() {
+        if (prev != device)
+            cudaSetDevice(prev);
+    }
+};
 
 } // namespace
 
@@ -225,6 +247,72 @@ void match(
     }
     if (prev != device)
         cudaSetDevice(prev);
+}
+
+void remap(const std::vector<Image>& src, const Image& map_x, const Image& map_y, std::vector<Image>& dst, void* stream) {
+    if (src.empty())
+        throw Exception("no images to remap");
+    const Image& first = src.front();
+    if (first.type() != IMG_8U && first.type() != IMG_16U)
+        throw Exception("bad input depths, only CV_8UC1 and CV_16UC1 are supported");
+    std::vector<const void*> planes;
+    for (const Image& im: src) {
+        if (im.empty() || im.rows != first.rows || im.cols != first.cols || im.type() != first.type() || im.step != first.step)
+            throw Exception("images to remap differ in size, type or pitch");
+        planes.push_back(im.data);
+    }
+    check_maps(map_x, map_y, map_x);
+    const int device = device_of(planes.front());
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    dst.resize(src.size());
+    std::vector<void*> out;
+    for (Image& im: dst) {
+        im.create(map_x.rows, map_x.cols, first.type());
+        out.push_back(im.data);
+    }
+    for (const Image& im: dst)
+        if (im.step != dst.front().step)
+            throw Exception("remap outputs differ in pitch");
+    const int rc = bicos_b200_remap(h, planes.data(), (int)planes.size(), first.rows, first.cols, first.step, first.depth(),
+                                    reinterpret_cast<const float*>(map_x.data), reinterpret_cast<const float*>(map_y.data),
+                                    map_x.step, map_x.rows, map_x.cols, out.data(), dst.front().step, stream);
+    if (rc != 0)
+        rethrow_last(rc);
+}
+
+void match_rectified(
+    const std::vector<Image>& stack0,
+    const std::vector<Image>& stack1,
+    const RectifyMaps& maps,
+    Image& disparity,
+    Config cfg,
+    Image* corrmap,
+    void* stream
+) {
+    const StackView v0 = view_of(stack0, "stack0");
+    const StackView v1 = view_of(stack1, "stack1");
+    if (stack0.size() != stack1.size() || v0.rows != v1.rows || v0.cols != v1.cols || v0.depth != v1.depth || v0.step != v1.step)
+        throw Exception("stack0 and stack1 differ in length, size, type or pitch");
+    check_maps(maps.map_x0, maps.map_y0, maps.map_x0);
+    check_maps(maps.map_x1, maps.map_y1, maps.map_x0);
+    const bicos_b200_config c = to_c_config(cfg);
+    const int device = device_of(v0.planes.front());
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    const int rows = maps.map_x0.rows, cols = maps.map_x0.cols;
+    disparity.create(rows, cols, bicos_b200_disparity_type(&c));
+    const bool want_corr = corrmap && cfg.nxcorr_threshold.has_value();
+    if (want_corr)
+        corrmap->create(rows, cols, bicos_b200_corrmap_type(&c));
+    const bicos_b200_rectify_maps m { reinterpret_cast<const float*>(maps.map_x0.data), reinterpret_cast<const float*>(maps.map_y0.data),
+                                      reinterpret_cast<const float*>(maps.map_x1.data), reinterpret_cast<const float*>(maps.map_y1.data),
+                                      maps.map_x0.step };
+    const int rc = bicos_b200_match_rectified(h, v0.planes.data(), v1.planes.data(), (int)stack0.size(), v0.rows, v0.cols, v0.step,
+                                              v0.depth, &m, rows, cols, &c, disparity.data, disparity.step,
+                                              want_corr ? corrmap->data : nullptr, want_corr ? corrmap->step : 0, stream);
+    if (rc != 0)
+        rethrow_last(rc);
 }
 
 void match_sharded(

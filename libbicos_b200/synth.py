@@ -168,3 +168,28 @@ def random_stacks(n, height, width, dtype=np.uint8, seed=1):
     a = rng.integers(0, hi, size=(n, height, width), dtype=np.int64).astype(dtype)
     b = rng.integers(0, hi, size=(n, height, width), dtype=np.int64).astype(dtype)
     return a, b
+
+
+def rectify_maps(rows, cols, src_rows=None, src_cols=None, camera=0, k1=-0.12, k2=0.03, angle_deg=0.6):
+    """Float32 rectification maps (map_x, map_y) [rows, cols] of a pinhole camera with radial distortion (k1, k2)
+    and a small rotation about the optical axis and the vertical axis, what cv2.initUndistortRectifyMap(K, D, R, P,
+    (cols, rows), CV_32FC1) computes: for a rectified pixel (u, v), the ray R^-1 P^-1 (u, v, 1), projected and
+    distorted into the source image of src_rows x src_cols (default: the rectified size). camera = 0 / 1 mirrors the
+    rotation, as the two cameras of a rig are rotated towards each other."""
+    src_rows = rows if src_rows is None else src_rows
+    src_cols = cols if src_cols is None else src_cols
+    f = 0.9 * max(src_rows, src_cols)
+    cx, cy = (src_cols - 1) / 2.0, (src_rows - 1) / 2.0
+    fn = 0.9 * max(rows, cols)  # P: the rectified camera
+    cxn, cyn = (cols - 1) / 2.0, (rows - 1) / 2.0
+    a = np.deg2rad(angle_deg) * (1 if camera == 0 else -1)
+    rz = np.array([[np.cos(a), -np.sin(a), 0], [np.sin(a), np.cos(a), 0], [0, 0, 1]])
+    b = 2 * a
+    ry = np.array([[np.cos(b), 0, np.sin(b)], [0, 1, 0], [-np.sin(b), 0, np.cos(b)]])
+    rinv = (rz @ ry).T
+    v, u = np.mgrid[0:rows, 0:cols].astype(np.float64)
+    ray = np.stack([(u - cxn) / fn, (v - cyn) / fn, np.ones_like(u)], axis=-1) @ rinv.T
+    x, y = ray[..., 0] / ray[..., 2], ray[..., 1] / ray[..., 2]
+    r2 = x * x + y * y
+    radial = 1 + k1 * r2 + k2 * r2 * r2
+    return (f * x * radial + cx).astype(np.float32), (f * y * radial + cy).astype(np.float32)
