@@ -1,4 +1,4 @@
-// BICOS::Image for builds without OpenCV: a reference-counted, pitched, single-channel
+// BICOS::Image for builds without OpenCV: a reference-counted, pitched
 // device matrix exposing the members of cv::cuda::GpuMat that callers of BICOS::match use
 // (rows, cols, step, data, type(), depth(), create(), upload(), download(), empty()).
 //
@@ -14,8 +14,10 @@
 
 namespace BICOS {
 
-// OpenCV type codes (single channel), so that code written against cv::Mat::type() keeps working
-constexpr int IMG_8U = 0, IMG_16U = 2, IMG_16S = 3, IMG_32F = 5, IMG_64F = 6;
+// OpenCV type codes, so that code written against cv::Mat::type() keeps working: single channel, plus the int32
+// pixel indices and the interleaved float32 X Y Z points of BICOS::reproject (reproject.hpp)
+constexpr int IMG_8U = 0, IMG_16U = 2, IMG_16S = 3, IMG_32S = 4, IMG_32F = 5, IMG_64F = 6;
+constexpr int IMG_32FC3 = 21; // CV_32FC3: depth IMG_32F, three channels (channel count - 1 in bits 3 and up)
 
 size_t image_elem_size(int type);
 
@@ -61,7 +63,7 @@ public:
         return type_ & 7;
     }
     int channels() const {
-        return 1;
+        return (type_ >> 3) + 1;
     }
     size_t elemSize() const {
         return image_elem_size(type_);

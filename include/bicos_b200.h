@@ -220,6 +220,42 @@ int bicos_b200_match_rectified(bicos_b200_handle h, const void* const* planes0, 
                                void* disparity, size_t disparity_pitch_bytes, void* corrmap, size_t corrmap_pitch_bytes,
                                void* stream);
 
+/* ---- reprojection: disparity out, 3D points out -----------------------------------------
+ * Turns a disparity map (of any match entry point) into 3D points through the 4x4 reprojection matrix Q of the
+ * rectified rig, e.g. the Q of OpenCV's cv::stereoRectify (computing Q is a host step and not part of this
+ * library). Semantics, bit for bit those of bicos-cli's point cloud, per disparity pixel (row r, column c) in
+ * row-major order:
+ *   skipped as invalid disparity: int16 -32768; float32 NaN or exactly -32768.0f (the marker of integer mode with
+ *   a threshold, see bicos_b200_match)
+ *   in = (c, r, d, 1.0) in double; o[k] = ((Q[4k] in0 + Q[4k+1] in1) + Q[4k+2] in2) + Q[4k+3] in3 for k = 0..3,
+ *   every product and every sum rounded to double on its own (no FMA contraction)
+ *   X = (float)(o0 / o3), Y = (float)(o1 / o3), Z = (float)(o2 / o3): IEEE division, correctly rounded; the
+ *   conversion rounds to nearest even and keeps subnormals
+ *   skipped as non-finite: X, Y or Z is +-inf or NaN (this includes W = o3 = 0 and values beyond the float range)
+ *   skipped as negative Z: Z < 0.0f (-0.0 is kept), unless BICOS_B200_REPROJECT_ALLOW_NEGATIVE_Z is set
+ *   kept: everything else
+ * This is not the arithmetic of OpenCV's cv::reprojectImageTo3D, which accumulates Q's columns incrementally,
+ * multiplies by 1/W and writes Z = 10000 for missing values; where both keep a point they agree within a few
+ * float ULPs. */
+#define BICOS_B200_REPROJECT_ALLOW_NEGATIVE_Z 1
+
+/* Stage entry point, one launch. disparity: device int16 (BICOS_B200_16S) or float32 (BICOS_B200_32F)
+ * [rows][disparity_pitch_bytes], pitch a multiple of the element size; rows and cols 1..32767. q: HOST array of
+ * 16 doubles, row-major. Outputs (device; at least one of xyz and points):
+ *   xyz          dense float32 [rows][xyz_pitch_bytes], X Y Z interleaved per pixel (pitch a multiple of 4 and at
+ *                least cols * 12), NaN NaN NaN for every skipped pixel; may be NULL
+ *   points       the kept points, float32 X Y Z (12 bytes each), densely packed in row-major pixel order: the
+ *                order and content of bicos-cli's .xyz file; capacity rows * cols points; may be NULL
+ *   pixel_index  int32 r * cols + c of each point, same order; capacity rows * cols; may be NULL, needs points
+ *   counts       device unsigned long long [4]: kept, invalid disparity, non-finite, negative Z; they sum to
+ *                rows * cols. Required with points (allowed with xyz alone). Only counts[0] entries of points
+ *                and pixel_index are written.
+ * Asynchronous. The call uses a workspace of the handle (grown on demand, freed by bicos_b200_destroy): a call on
+ * another stream than the handle's previous work first waits for that work, as a match does. */
+int bicos_b200_reproject(bicos_b200_handle h, const void* disparity, int disparity_type, size_t disparity_pitch_bytes,
+                         int rows, int cols, const double q[16], int flags, float* xyz, size_t xyz_pitch_bytes,
+                         float* points, int32_t* pixel_index, unsigned long long* counts, void* stream);
+
 /* Throughput mode: `count` independent stereo stacks of one shape, type and configuration (BASELINE.json's batch
  * configuration). planes0[f] / planes1[f] are the n plane pointers of frame f, disparity[f] / corrmap[f] its outputs
  * (corrmap may be NULL, or hold NULL entries). Same results as `count` calls of bicos_b200_match, but the frames

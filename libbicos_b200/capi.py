@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_PKG, "libbicos_b200.so")
 
 DEPTH_8U, DEPTH_16U, TYPE_16S, TYPE_32F, TYPE_64F = 0, 2, 3, 5, 6
 FLAG_NODUPES, FLAG_CONSISTENCY, FLAG_TOP_BIT_FREE, FLAG_TOP2_BITS_FREE = 1, 2, 4, 8
+REPROJECT_ALLOW_NEGATIVE_Z = 1
 MAX_IMAGES = 65
 
 EXPORTS = (
@@ -27,7 +28,7 @@ EXPORTS = (
     "bicos_b200_kernel_launches", "bicos_b200_set_profiling", "bicos_b200_stage_times",
     "bicos_b200_shared_alloc", "bicos_b200_shared_open", "bicos_b200_shared_close", "bicos_b200_shared_free",
     "bicos_b200_set_search_engine", "bicos_b200_get_search_engine", "bicos_b200_last_search_kernel",
-    "bicos_b200_remap", "bicos_b200_match_rectified",
+    "bicos_b200_remap", "bicos_b200_match_rectified", "bicos_b200_reproject",
 )
 SEARCH_ENGINES = {"auto": 0, "popc": 1, "tensor": 2}
 IPC_HANDLE_BYTES = 64
@@ -159,6 +160,7 @@ def lib():
         L.bicos_b200_remap.argtypes = [vp, pp, i, i, i, sz, i, vp, vp, sz, i, i, pp, sz, vp]
         L.bicos_b200_match_rectified.argtypes = [vp, pp, pp, i, i, i, sz, i, ctypes.POINTER(CRectifyMaps), i, i, cfgp, vp, sz, vp,
                                                  sz, vp]
+        L.bicos_b200_reproject.argtypes = [vp, vp, i, sz, i, i, ctypes.POINTER(ctypes.c_double), i, vp, sz, vp, vp, vp, vp]
         L.bicos_b200_stage_times.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_longlong)]
         _lib = L
     return _lib
@@ -451,6 +453,69 @@ class Handle:
             disp.data_ptr(), disp.stride(0) * disp.element_size(), corr.data_ptr() if corr is not None else None,
             corr.stride(0) * corr.element_size() if corr is not None else 0, self._stream()))
         return disp, corr
+
+    @staticmethod
+    def _disparity_info(disparity):
+        """(type code, rows, cols, pitch in bytes) of an int16 / float32 CUDA tensor [rows, cols] with contiguous rows."""
+        import torch
+
+        if not isinstance(disparity, torch.Tensor) or disparity.dim() != 2 or not disparity.is_cuda:
+            raise BicosError("the disparity must be a CUDA tensor of shape [rows, cols]")
+        codes = {torch.int16: TYPE_16S, torch.float32: TYPE_32F}
+        if disparity.dtype not in codes:
+            raise BicosError("the disparity must be int16 or float32")
+        if disparity.stride(1) != 1:
+            raise BicosError("disparity rows must be contiguous")
+        rows, cols = disparity.shape
+        return codes[disparity.dtype], rows, cols, disparity.stride(0) * disparity.element_size()
+
+    @staticmethod
+    def _q_matrix(Q):
+        """Q as the 16 row-major float64 values the C ABI takes from host memory."""
+        import numpy as np
+
+        if hasattr(Q, "detach"):
+            Q = Q.detach().cpu().numpy()
+        q = np.ascontiguousarray(np.asarray(Q, dtype=np.float64))
+        if q.shape != (4, 4):
+            raise BicosError(f"Q must be 4 x 4, got shape {q.shape}")
+        return (ctypes.c_double * 16)(*q.ravel().tolist())
+
+    def reproject(self, disparity, Q, allow_negative_z: bool = False, out=None):
+        """Dense reprojection (bicos_b200_reproject): [rows, cols] int16 / float32 CUDA disparity -> [rows, cols, 3]
+        float32 X Y Z, NaN where a pixel is skipped (invalid disparity, non-finite point, Z < 0 unless
+        ``allow_negative_z``); include/bicos_b200.h states the arithmetic. ``Q``: any 4 x 4 array-like. ``out``: a
+        float32 tensor [rows, cols, 3] on the disparity's device with contiguous pixels."""
+        import torch
+
+        code, rows, cols, pitch = self._disparity_info(disparity)
+        if out is None:
+            out = torch.empty((rows, cols, 3), dtype=torch.float32, device=disparity.device)
+        elif (not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or tuple(out.shape) != (rows, cols, 3)
+              or out.device != disparity.device or out.stride(2) != 1 or out.stride(1) != 3):
+            raise BicosError(f"out must be a float32 tensor of shape ({rows}, {cols}, 3) on {disparity.device} with contiguous rows")
+        _check(lib().bicos_b200_reproject(self._h, disparity.data_ptr(), code, pitch, rows, cols, self._q_matrix(Q),
+                                          REPROJECT_ALLOW_NEGATIVE_Z if allow_negative_z else 0, out.data_ptr(), out.stride(0) * 4,
+                                          None, None, None, self._stream()))
+        return out
+
+    def reproject_points(self, disparity, Q, allow_negative_z: bool = False):
+        """The kept points of reproject() in row-major pixel order -> (points [N, 3] float32, pixel_index [N] int32 =
+        row * cols + col, counts), counts = {"points", "invalid_disparity", "non_finite", "negative_z"} summing to
+        rows * cols. Synchronises the current stream to learn N; the tensors are views of rows * cols capacity."""
+        import torch
+
+        code, rows, cols, pitch = self._disparity_info(disparity)
+        dev = disparity.device
+        points = torch.empty((rows * cols, 3), dtype=torch.float32, device=dev)
+        index = torch.empty((rows * cols,), dtype=torch.int32, device=dev)
+        counts = torch.empty((4,), dtype=torch.int64, device=dev)
+        _check(lib().bicos_b200_reproject(self._h, disparity.data_ptr(), code, pitch, rows, cols, self._q_matrix(Q),
+                                          REPROJECT_ALLOW_NEGATIVE_Z if allow_negative_z else 0, None, 0, points.data_ptr(),
+                                          index.data_ptr(), counts.data_ptr(), self._stream()))
+        kept, invalid, non_finite, negative_z = (int(v) for v in counts.cpu().tolist())
+        return points[:kept], index[:kept], dict(points=kept, invalid_disparity=invalid, non_finite=non_finite,
+                                                 negative_z=negative_z)
 
     def match_batch(self, frames, cfg: Config, outs=None):
         """Throughput mode (bicos_b200_match_batch): `frames` = [(stack0, stack1), ...] of one shape and dtype,

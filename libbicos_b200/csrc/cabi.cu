@@ -303,6 +303,7 @@ struct bicos_b200_handle_s {
     DeviceBuffer desc0, desc1, keys, xs; // keys: up to four [rows][cols] uint32 search-key arrays
     DeviceBuffer stage_in, stage_disp, stage_corr;
     DeviceBuffer rect; // bicos_b200_match_rectified: both rectified stacks, [2n][rows][rect pitch]
+    DeviceBuffer reproj; // bicos_b200_reproject: ReprojectWork + one look-back status word per tile
     float xs_step = -1.f;
     int xs_count = 0;
     bool host_pending = false; // between bicos_b200_match_host_begin and _end
@@ -790,7 +791,7 @@ int bicos_b200_destroy(bicos_b200_handle h) {
     {
         DeviceGuard g(h->device);
         cudaDeviceSynchronize();
-        for (DeviceBuffer* b: { &h->desc0, &h->desc1, &h->keys, &h->xs, &h->stage_in, &h->stage_disp, &h->stage_corr, &h->rect })
+        for (DeviceBuffer* b: { &h->desc0, &h->desc1, &h->keys, &h->xs, &h->stage_in, &h->stage_disp, &h->stage_corr, &h->rect, &h->reproj })
             b->release();
         for (cudaEvent_t e: h->prof_events)
             cudaEventDestroy(e);
@@ -1120,6 +1121,65 @@ int bicos_b200_match_rectified(bicos_b200_handle h, const void* const* planes0, 
     }
     return match_banded_or_whole(h, rect0.data(), rect1.data(), n, rows, cols, pitch, depth, cfg, disparity, disparity_pitch_bytes,
                                  corrmap, corrmap_pitch_bytes, s);
+}
+
+int bicos_b200_reproject(bicos_b200_handle h, const void* disparity, int disparity_type, size_t disparity_pitch_bytes,
+                         int rows, int cols, const double q[16], int flags, float* xyz, size_t xyz_pitch_bytes,
+                         float* points, int32_t* pixel_index, unsigned long long* counts, void* stream) {
+    if (!h || !q || !disparity)
+        return fail(BICOS_B200_ERR_INVALID, "null argument");
+    if (disparity_type != BICOS_B200_16S && disparity_type != BICOS_B200_32F)
+        return fail(BICOS_B200_ERR_INVALID, "bad disparity type %d: only int16 (CV_16SC1) and float32 (CV_32FC1)", disparity_type);
+    if ((flags & ~BICOS_B200_REPROJECT_ALLOW_NEGATIVE_Z) != 0)
+        return fail(BICOS_B200_ERR_INVALID, "unknown reprojection flags %#x", flags);
+    if (!xyz && !points)
+        return fail(BICOS_B200_ERR_INVALID, "no output: give xyz, points, or both");
+    if (points && !counts)
+        return fail(BICOS_B200_ERR_INVALID, "points need counts");
+    if (pixel_index && !points)
+        return fail(BICOS_B200_ERR_INVALID, "pixel_index needs points");
+    if (rows < 1 || cols < 1 || rows > 32767 || cols > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "disparity of %d x %d: rows and cols must be 1 to 32767", rows, cols);
+    const size_t es = disparity_type == BICOS_B200_16S ? 2 : 4;
+    if (disparity_pitch_bytes < (size_t)cols * es || disparity_pitch_bytes % es != 0 || reinterpret_cast<uintptr_t>(disparity) % es != 0)
+        return fail(BICOS_B200_ERR_INVALID, "disparity rows must be aligned to and hold cols elements");
+    if (xyz && (xyz_pitch_bytes < (size_t)cols * 3 * sizeof(float) || xyz_pitch_bytes % sizeof(float) != 0 ||
+                reinterpret_cast<uintptr_t>(xyz) % sizeof(float) != 0))
+        return fail(BICOS_B200_ERR_INVALID, "xyz rows must be 4-byte aligned and hold cols * 3 float32 values");
+    if ((points && reinterpret_cast<uintptr_t>(points) % sizeof(float) != 0) ||
+        (pixel_index && reinterpret_cast<uintptr_t>(pixel_index) % sizeof(int32_t) != 0) ||
+        (counts && reinterpret_cast<uintptr_t>(counts) % sizeof(unsigned long long) != 0))
+        return fail(BICOS_B200_ERR_INVALID, "misaligned points, pixel_index or counts");
+    DeviceGuard g(h->device);
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    ReprojectParams prm {};
+    prm.disparity = disparity;
+    prm.disparity_pitch = disparity_pitch_bytes;
+    prm.rows = rows;
+    prm.cols = cols;
+    for (int k = 0; k < 16; ++k)
+        prm.q[k] = q[k];
+    prm.allow_negative_z = (flags & BICOS_B200_REPROJECT_ALLOW_NEGATIVE_Z) ? 1 : 0;
+    prm.xyz = xyz;
+    prm.xyz_pitch = xyz_pitch_bytes;
+    prm.points = points;
+    prm.pixel_index = pixel_index;
+    prm.counts = counts;
+    if (int rc = enter_workspace(h, s)) // the previous call of the handle may still use the status words
+        return rc;
+    if (counts) {
+        const size_t work_bytes = sizeof(ReprojectWork) + sizeof(unsigned long long) * (size_t)reproject_tiles(rows, cols);
+        CU(h->reproj.reserve(work_bytes));
+        CU(cudaMemsetAsync(h->reproj.ptr, 0, work_bytes, s));
+        prm.work = static_cast<ReprojectWork*>(h->reproj.ptr);
+        prm.status = reinterpret_cast<unsigned long long*>(prm.work + 1);
+    }
+    {
+        Range nvtx("bicos_b200::reproject");
+        CU(launch_reproject(prm, disparity_type == BICOS_B200_32F, s));
+        h->launches += 1;
+    }
+    return leave_workspace(h, s);
 }
 
 int bicos_b200_match_rows(bicos_b200_handle h, const void* const* planes0,

@@ -209,4 +209,32 @@ struct RemapParams {
 // `sides` = 1 or 2: blockIdx.z picks prm.side[z], so both stacks of a match are one launch
 cudaError_t launch_remap(const RemapParams& prm, int sides, int is_u16, cudaStream_t stream);
 
+// stage 4 (reproject.cu): disparity -> 3D points through Q with the arithmetic bicos_b200_reproject states. One
+// launch writes the dense map `xyz` and / or the ordered point list (`points`, `pixel_index`) with `counts`.
+// The list and the counters need `work` and `status` zeroed before the launch (one cudaMemsetAsync of
+// sizeof(ReprojectWork) + reproject_tiles() status words); a dense map alone runs without them.
+struct ReprojectWork {
+    unsigned int ticket; // next tile to hand out
+    unsigned int done; // CTAs that have added their counters
+    unsigned long long count[4]; // kept, invalid disparity, non-finite, negative Z
+};
+
+struct ReprojectParams {
+    const void* disparity; // int16 or float32 [rows][disparity_pitch bytes]
+    size_t disparity_pitch;
+    int rows, cols; // 1 .. 32767
+    double q[16]; // row-major
+    int allow_negative_z;
+    float* xyz; // [rows][xyz_pitch bytes], 3 floats per pixel; may be null
+    size_t xyz_pitch;
+    float* points; // [rows * cols][3]; may be null
+    int32_t* pixel_index; // [rows * cols]; may be null
+    unsigned long long* counts; // [4]; required with points
+    ReprojectWork* work; // required with points or counts
+    unsigned long long* status; // [reproject_tiles()] look-back status words, after `work`
+};
+
+int reproject_tiles(int rows, int cols);
+cudaError_t launch_reproject(const ReprojectParams& prm, int is_float, cudaStream_t stream);
+
 } // namespace bicos_b200

@@ -4,6 +4,7 @@
 
 #include "../../include/BICOS/match.hpp"
 #include "../../include/BICOS/rectify.hpp"
+#include "../../include/BICOS/reproject.hpp"
 #include "../../include/bicos_b200.h"
 
 #include <cuda_runtime.h>
@@ -34,7 +35,12 @@ void cuda_check(cudaError_t err, const char* what) {
 // reference (which has no global mutable state), and repeated calls reuse their buffers.
 struct HandleCache {
     std::map<int, bicos_b200_handle> handles;
+    std::map<int, unsigned long long*> counts; // reproject_points: the four device counters
     ~HandleCache() {
+        for (auto& kv: counts) {
+            cudaSetDevice(kv.first);
+            cudaFree(kv.second);
+        }
         for (auto& kv: handles)
             bicos_b200_destroy(kv.second);
     }
@@ -52,6 +58,17 @@ struct HandleCache {
 };
 
 thread_local HandleCache t_handles;
+
+// the device counters of reproject_points on `device` (current)
+unsigned long long* counts_buffer(int device) {
+    auto it = t_handles.counts.find(device);
+    if (it != t_handles.counts.end())
+        return it->second;
+    void* p = nullptr;
+    cuda_check(cudaMalloc(&p, 4 * sizeof(unsigned long long)), "cudaMalloc");
+    t_handles.counts[device] = static_cast<unsigned long long*>(p);
+    return static_cast<unsigned long long*>(p);
+}
 
 bicos_b200_config to_c_config(const Config& cfg) {
     bicos_b200_config c {};
@@ -138,6 +155,8 @@ struct DeviceScope {
 } // namespace
 
 size_t image_elem_size(int type) {
+    if (type == IMG_32FC3)
+        return 3 * sizeof(float);
     switch (type & 7) {
         case IMG_8U:
         case 1:
@@ -313,6 +332,54 @@ void match_rectified(
                                               want_corr ? corrmap->data : nullptr, want_corr ? corrmap->step : 0, stream);
     if (rc != 0)
         rethrow_last(rc);
+}
+
+namespace {
+
+void check_disparity(const Image& disparity) {
+    if (disparity.empty() || (disparity.type() != IMG_16S && disparity.type() != IMG_32F))
+        throw Exception("reprojection needs a non-empty CV_16SC1 or CV_32FC1 disparity image");
+}
+
+} // namespace
+
+void reproject(const Image& disparity, const std::array<double, 16>& Q, Image& xyz, bool allow_negative_z, void* stream) {
+    check_disparity(disparity);
+    const int device = device_of(disparity.data);
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    xyz.create(disparity.rows, disparity.cols, IMG_32FC3);
+    const int rc = bicos_b200_reproject(h, disparity.data, disparity.type(), disparity.step, disparity.rows, disparity.cols, Q.data(),
+                                        allow_negative_z ? BICOS_B200_REPROJECT_ALLOW_NEGATIVE_Z : 0,
+                                        reinterpret_cast<float*>(xyz.data), xyz.step, nullptr, nullptr, nullptr, stream);
+    if (rc != 0)
+        rethrow_last(rc);
+}
+
+ReprojectCounts reproject_points(const Image& disparity, const std::array<double, 16>& Q, Image& points, Image* pixel_index,
+                                 bool allow_negative_z, void* stream) {
+    check_disparity(disparity);
+    const int device = device_of(disparity.data);
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    if (disparity.rows > 32767 || disparity.cols > 32767)
+        throw Exception("reprojection: the disparity has more than 32767 rows or columns");
+    const int capacity = disparity.rows * disparity.cols; // < 2^30
+    points.create(1, capacity, IMG_32FC3);
+    if (pixel_index)
+        pixel_index->create(1, capacity, IMG_32S);
+    unsigned long long* counts = counts_buffer(device);
+    const int rc = bicos_b200_reproject(h, disparity.data, disparity.type(), disparity.step, disparity.rows, disparity.cols, Q.data(),
+                                        allow_negative_z ? BICOS_B200_REPROJECT_ALLOW_NEGATIVE_Z : 0, nullptr, 0,
+                                        reinterpret_cast<float*>(points.data),
+                                        pixel_index ? reinterpret_cast<int32_t*>(pixel_index->data) : nullptr, counts, stream);
+    if (rc != 0)
+        rethrow_last(rc);
+    unsigned long long host[4] = { 0, 0, 0, 0 };
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    cuda_check(cudaMemcpyAsync(host, counts, sizeof host, cudaMemcpyDeviceToHost, s), "download counts");
+    cuda_check(cudaStreamSynchronize(s), "cudaStreamSynchronize");
+    return ReprojectCounts { (size_t)host[0], (size_t)host[1], (size_t)host[2], (size_t)host[3] };
 }
 
 void match_sharded(
