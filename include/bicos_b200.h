@@ -256,6 +256,33 @@ int bicos_b200_reproject(bicos_b200_handle h, const void* disparity, int dispari
                          int rows, int cols, const double q[16], int flags, float* xyz, size_t xyz_pitch_bytes,
                          float* points, int32_t* pixel_index, unsigned long long* counts, void* stream);
 
+/* ---- speckle removal: disparity in, disparity out, in place ---------------------------------
+ * Sets small connected blobs of a disparity map to `new_value`, like OpenCV's cv::filterSpeckles(img, newVal,
+ * maxSpeckleSize, maxDiff), whose parameters come in the same order. disparity: device int16 (BICOS_B200_16S) or
+ * float32 (BICOS_B200_32F) [rows][disparity_pitch_bytes], pitch a multiple of the element size; rows and cols
+ * 1..32767. Semantics:
+ *   parameters: int16: new = cvRound(new_value), diff = cvRound(max_diff), both rounded half to even; `new` outside
+ *   int16 is BICOS_B200_ERR_INVALID; a diff beyond +-65535 acts as +-65535. float32: new = (float)new_value (NaN
+ *   allowed), diff = (float)max_diff. A NaN max_diff is BICOS_B200_ERR_INVALID.
+ *   members: pixels that are not an invalid marker (int16 -32768; float32 NaN or -32768.0f: the pixels
+ *   bicos_b200_reproject skips) and not equal to `new`
+ *   edges: two 4-neighbours are connected when both are members and |d(p) - d(q)| <= diff; int16 computes the
+ *   difference in int32, float32 compares fabsf of the float32 difference rounded to nearest (no contraction), so
+ *   inf - inf (NaN) gives no edge
+ *   speckles: connected components of at most max_speckle_size members; every pixel of a speckle is set to `new`.
+ *   Nothing else is written, the pitch padding included. max_speckle_size <= 0 changes nothing; a negative diff
+ *   makes every member a component of its own.
+ *   counts (optional, device unsigned long long [2], 8-byte aligned): the pixels set and the speckles removed.
+ * For int16 with new_value = -32768, or with no -32768 pixels, the result is exactly cv::filterSpeckles' (for
+ * diff <= 32767: OpenCV's IPP path truncates a larger maxDiff to int16, its plain path does not). The
+ * deliberate differences: float32 is supported, and markers are never members whatever new_value is.
+ * Asynchronous; four launches on every input, whatever its content. The call uses a workspace of the handle (8
+ * bytes per pixel, grown on demand, freed by bicos_b200_destroy): a call on another stream than the handle's
+ * previous work first waits for that work, as a match does. */
+int bicos_b200_filter_speckles(bicos_b200_handle h, void* disparity, int disparity_type, size_t disparity_pitch_bytes, int rows,
+                               int cols, double new_value, int max_speckle_size, double max_diff, unsigned long long* counts,
+                               void* stream);
+
 /* Throughput mode: `count` independent stereo stacks of one shape, type and configuration (BASELINE.json's batch
  * configuration). planes0[f] / planes1[f] are the n plane pointers of frame f, disparity[f] / corrmap[f] its outputs
  * (corrmap may be NULL, or hold NULL entries). Same results as `count` calls of bicos_b200_match, but the frames

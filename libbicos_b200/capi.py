@@ -28,7 +28,7 @@ EXPORTS = (
     "bicos_b200_kernel_launches", "bicos_b200_set_profiling", "bicos_b200_stage_times",
     "bicos_b200_shared_alloc", "bicos_b200_shared_open", "bicos_b200_shared_close", "bicos_b200_shared_free",
     "bicos_b200_set_search_engine", "bicos_b200_get_search_engine", "bicos_b200_last_search_kernel",
-    "bicos_b200_remap", "bicos_b200_match_rectified", "bicos_b200_reproject",
+    "bicos_b200_remap", "bicos_b200_match_rectified", "bicos_b200_reproject", "bicos_b200_filter_speckles",
 )
 SEARCH_ENGINES = {"auto": 0, "popc": 1, "tensor": 2}
 IPC_HANDLE_BYTES = 64
@@ -161,6 +161,7 @@ def lib():
         L.bicos_b200_match_rectified.argtypes = [vp, pp, pp, i, i, i, sz, i, ctypes.POINTER(CRectifyMaps), i, i, cfgp, vp, sz, vp,
                                                  sz, vp]
         L.bicos_b200_reproject.argtypes = [vp, vp, i, sz, i, i, ctypes.POINTER(ctypes.c_double), i, vp, sz, vp, vp, vp, vp]
+        L.bicos_b200_filter_speckles.argtypes = [vp, vp, i, sz, i, i, ctypes.c_double, i, ctypes.c_double, vp, vp]
         L.bicos_b200_stage_times.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_longlong)]
         _lib = L
     return _lib
@@ -516,6 +517,24 @@ class Handle:
         kept, invalid, non_finite, negative_z = (int(v) for v in counts.cpu().tolist())
         return points[:kept], index[:kept], dict(points=kept, invalid_disparity=invalid, non_finite=non_finite,
                                                  negative_z=negative_z)
+
+    def filter_speckles(self, disparity, new_value, max_speckle_size: int, max_diff, counts: bool = False):
+        """Speckle removal in place (bicos_b200_filter_speckles, cv::filterSpeckles' parameters in its order) on a
+        [rows, cols] int16 / float32 CUDA disparity: every connected blob of at most ``max_speckle_size`` valid pixels
+        whose 4-neighbours differ by at most ``max_diff`` is set to ``new_value``; include/bicos_b200.h states the
+        semantics. Returns the tensor, or with ``counts`` (tensor, {"pixels", "speckles"}): the pixels set and the
+        speckles removed, which synchronises the current stream. Without ``counts`` nothing synchronises."""
+        import torch
+
+        code, rows, cols, pitch = self._disparity_info(disparity)
+        dev_counts = torch.empty((2,), dtype=torch.int64, device=disparity.device) if counts else None
+        _check(lib().bicos_b200_filter_speckles(self._h, disparity.data_ptr(), code, pitch, rows, cols, float(new_value),
+                                                int(max_speckle_size), float(max_diff),
+                                                dev_counts.data_ptr() if counts else None, self._stream()))
+        if not counts:
+            return disparity
+        pixels, speckles = (int(v) for v in dev_counts.cpu().tolist())
+        return disparity, dict(pixels=pixels, speckles=speckles)
 
     def match_batch(self, frames, cfg: Config, outs=None):
         """Throughput mode (bicos_b200_match_batch): `frames` = [(stack0, stack1), ...] of one shape and dtype,

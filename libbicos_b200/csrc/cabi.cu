@@ -304,6 +304,7 @@ struct bicos_b200_handle_s {
     DeviceBuffer stage_in, stage_disp, stage_corr;
     DeviceBuffer rect; // bicos_b200_match_rectified: both rectified stacks, [2n][rows][rect pitch]
     DeviceBuffer reproj; // bicos_b200_reproject: ReprojectWork + one look-back status word per tile
+    DeviceBuffer speckle; // bicos_b200_filter_speckles: union-find parents and component sizes, int32 [2][rows * cols]
     float xs_step = -1.f;
     int xs_count = 0;
     bool host_pending = false; // between bicos_b200_match_host_begin and _end
@@ -791,7 +792,8 @@ int bicos_b200_destroy(bicos_b200_handle h) {
     {
         DeviceGuard g(h->device);
         cudaDeviceSynchronize();
-        for (DeviceBuffer* b: { &h->desc0, &h->desc1, &h->keys, &h->xs, &h->stage_in, &h->stage_disp, &h->stage_corr, &h->rect, &h->reproj })
+        for (DeviceBuffer* b: { &h->desc0, &h->desc1, &h->keys, &h->xs, &h->stage_in, &h->stage_disp, &h->stage_corr, &h->rect, &h->reproj,
+                                &h->speckle })
             b->release();
         for (cudaEvent_t e: h->prof_events)
             cudaEventDestroy(e);
@@ -1178,6 +1180,58 @@ int bicos_b200_reproject(bicos_b200_handle h, const void* disparity, int dispari
         Range nvtx("bicos_b200::reproject");
         CU(launch_reproject(prm, disparity_type == BICOS_B200_32F, s));
         h->launches += 1;
+    }
+    return leave_workspace(h, s);
+}
+
+int bicos_b200_filter_speckles(bicos_b200_handle h, void* disparity, int disparity_type, size_t disparity_pitch_bytes, int rows,
+                               int cols, double new_value, int max_speckle_size, double max_diff, unsigned long long* counts,
+                               void* stream) {
+    if (!h || !disparity)
+        return fail(BICOS_B200_ERR_INVALID, "null argument");
+    if (disparity_type != BICOS_B200_16S && disparity_type != BICOS_B200_32F)
+        return fail(BICOS_B200_ERR_INVALID, "bad disparity type %d: only int16 (CV_16SC1) and float32 (CV_32FC1)", disparity_type);
+    if (rows < 1 || cols < 1 || rows > 32767 || cols > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "disparity of %d x %d: rows and cols must be 1 to 32767", rows, cols);
+    const size_t es = disparity_type == BICOS_B200_16S ? 2 : 4;
+    if (disparity_pitch_bytes < (size_t)cols * es || disparity_pitch_bytes % es != 0 || reinterpret_cast<uintptr_t>(disparity) % es != 0)
+        return fail(BICOS_B200_ERR_INVALID, "disparity rows must be aligned to and hold cols elements");
+    if (std::isnan(max_diff))
+        return fail(BICOS_B200_ERR_INVALID, "max_diff is NaN");
+    if (counts && reinterpret_cast<uintptr_t>(counts) % sizeof(unsigned long long) != 0)
+        return fail(BICOS_B200_ERR_INVALID, "misaligned counts");
+    SpeckleParams prm {};
+    if (disparity_type == BICOS_B200_16S) {
+        // cvRound: to nearest, half to even (the default rounding mode)
+        const double nv = std::nearbyint(new_value), nd = std::nearbyint(max_diff);
+        if (!(nv >= -32768.0 && nv <= 32767.0))
+            return fail(BICOS_B200_ERR_INVALID, "new_value %g does not round into int16", new_value);
+        prm.new_i = (int)nv;
+        prm.diff_i = (int)std::fmax(-65535.0, std::fmin(65535.0, nd)); // int16 differences lie within +-65535
+    } else {
+        prm.new_f = (float)new_value;
+        prm.diff_f = (float)max_diff;
+    }
+    prm.disparity = disparity;
+    prm.disparity_pitch = disparity_pitch_bytes;
+    prm.rows = rows;
+    prm.cols = cols;
+    prm.max_size = max_speckle_size;
+    prm.counts = counts;
+    DeviceGuard g(h->device);
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (int rc = enter_workspace(h, s)) // the previous call of the handle may still use the labels
+        return rc;
+    const size_t px = (size_t)rows * cols;
+    CU(h->speckle.reserve(2 * px * sizeof(int)));
+    prm.parent = static_cast<int*>(h->speckle.ptr);
+    prm.size = prm.parent + px;
+    if (counts)
+        CU(cudaMemsetAsync(counts, 0, 2 * sizeof(unsigned long long), s));
+    {
+        Range nvtx("bicos_b200::filter_speckles");
+        CU(launch_speckles(prm, disparity_type == BICOS_B200_32F, s));
+        h->launches += 4;
     }
     return leave_workspace(h, s);
 }

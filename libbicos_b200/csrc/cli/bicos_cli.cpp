@@ -1,11 +1,12 @@
 // bicos-cli on the B200 path: same options, defaults and outputs as the reference CLI
 // (reference src/cli.cpp:55-253), without its dependencies (cxxopts, fmt, OpenCV): the argument
 // parser and the image I/O (imageio.cpp) are self-contained, the matching is BICOS::match from
-// include/BICOS/match.hpp and the point cloud of -q is BICOS::reproject_points from include/BICOS/reproject.hpp.
+// include/BICOS/match.hpp, the point cloud of -q is BICOS::reproject_points from include/BICOS/reproject.hpp and
+// --speckles is BICOS::filter_speckles from include/BICOS/speckles.hpp.
 //
 //   bicos-cli folder0 [folder1] [-t thr] [-v var] [-s step] [-o out.png] [-n N] [-q Q.yaml]
 //             [--allow-negative-z] [-m lr-maxdiff] [--double] [--limited] [--corrmap] [--no-dupes] [--wide-descriptors]
-//             [--disparity-range MIN:MAX]
+//             [--disparity-range MIN:MAX] [--speckles SIZE:DIFF]
 //
 // Differences, on purpose: --allow-negative-z is honoured (the reference reads a non-existent
 // "allow-behind" option, cli.cpp:231); integer-mode disparities with a threshold are float32
@@ -13,6 +14,7 @@
 // library follows) and are masked as invalid in the outputs.
 #include <BICOS/match.hpp>
 #include <BICOS/reproject.hpp>
+#include <BICOS/speckles.hpp>
 
 #include "imageio.hpp"
 
@@ -65,6 +67,7 @@ const Option OPTIONS[] = {
     { "no-dupes", 0, false, "Default BICOS variant when --lr-maxdiff is not specified. Can be set together with --lr-maxdiff to activate both." },
     { "wide-descriptors", 0, false, "Extension: accept 17..23 images without --limited (384 / 512-bit descriptors; the reference stops at 16)." },
     { "disparity-range", 0, true, "Extension: search only disparities MIN..MAX (inclusive, may be negative), e.g. 0:127. (default: the whole row)" },
+    { "speckles", 0, true, "Extension: after the match, mark connected blobs of at most SIZE pixels whose neighbours differ by at most DIFF as invalid, e.g. 100:1. (default: off)" },
     { "help", 'h', false, "Display this message." },
 };
 
@@ -342,6 +345,25 @@ int run(int argc, char const* const* argv) {
     }
     if (args.has("lr-maxdiff"))
         c.variant = Variant::Consistency { (int)to_uint(args, "lr-maxdiff"), args.has("no-dupes") };
+    std::optional<std::pair<int, double>> speckles;
+    if (args.has("speckles")) {
+        const std::string& v = args.get("speckles");
+        const size_t colon = v.find(':');
+        size_t used0 = 0, used1 = 0;
+        int size = 0;
+        double diff = 0.0;
+        try {
+            if (colon == std::string::npos)
+                throw std::invalid_argument("no colon");
+            size = std::stoi(v.substr(0, colon), &used0);
+            diff = std::stod(v.substr(colon + 1), &used1);
+        } catch (const std::exception&) {
+            used0 = 0;
+        }
+        if (used0 == 0 || used0 != colon || used1 == 0 || used1 != v.size() - colon - 1 || std::isnan(diff))
+            throw std::invalid_argument("Option 'speckles' expects SIZE:DIFF, got '" + v + "'");
+        speckles = std::make_pair(size, diff);
+    }
 
     auto tick = std::chrono::high_resolution_clock::now();
     std::vector<Image> lstack = upload(lseq), rstack = upload(rseq);
@@ -351,10 +373,17 @@ int run(int argc, char const* const* argv) {
     Image disp_gpu, corr_gpu;
     tick = std::chrono::high_resolution_clock::now();
     BICOS::match(lstack, rstack, disp_gpu, c, need_corrmap ? &corr_gpu : nullptr);
+    SpeckleCounts removed {};
+    if (speckles) {
+        // speckles become the type's invalid marker, so the masking below applies unchanged: int16 -32768; float32 NaN
+        // in subpixel mode and -32768.0f in integer mode; the corrmap is left as the match wrote it
+        const double marker = disp_gpu.type() == IMG_32F && c.subpixel_step.value_or(-1.f) >= 0.f ? std::nan("") : -32768.0;
+        filter_speckles(disp_gpu, marker, speckles->first, speckles->second, &removed);
+    }
     // the reference's match() returns after its work is done (its destructors synchronise):
     // download() below synchronises the default stream, so time that part with the match
     std::vector<uint8_t> disp = download(disp_gpu);
-    std::printf("%gms (match + disparity download)\t", ms_since(tick));
+    std::printf("%gms (match%s + disparity download)\t", ms_since(tick), speckles ? " + speckles" : "");
     std::fflush(stdout);
 
     tick = std::chrono::high_resolution_clock::now();
@@ -363,6 +392,8 @@ int run(int argc, char const* const* argv) {
         corrmap = download(corr_gpu);
     std::printf("%gms (download)\n", ms_since(tick));
 
+    if (speckles)
+        std::printf("Removed %zu speckles (%zu pixels)\n", removed.speckles, removed.pixels);
     const int rows = disp_gpu.rows, cols = disp_gpu.cols;
     save_image(disp, disp_gpu.type(), rows, cols, outfile, Colormap::TURBO);
     if (need_corrmap && !corrmap.empty())

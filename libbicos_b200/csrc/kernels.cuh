@@ -237,4 +237,22 @@ struct ReprojectParams {
 int reproject_tiles(int rows, int cols);
 cudaError_t launch_reproject(const ReprojectParams& prm, int is_float, cudaStream_t stream);
 
+// speckle removal (speckles.cu): in place on an int16 or float32 disparity with the semantics
+// bicos_b200_filter_speckles states. Four launches on every input (tile labelling, border merge, flatten and size,
+// write); `parent` and `size` are rows * cols int32 each and need no initialisation, `counts` ([2]: pixels set,
+// speckles removed) is added to and must be zeroed before the launch.
+struct SpeckleParams {
+    void* disparity; // int16 or float32 [rows][disparity_pitch bytes], written in place
+    size_t disparity_pitch;
+    int rows, cols; // 1 .. 32767
+    int new_i, diff_i; // int16: the converted new_value and max_diff
+    float new_f, diff_f; // float32: the same
+    int max_size; // components of at most this many members are speckles
+    int* parent; // [rows * cols] union-find parents (pixel indices)
+    int* size; // [rows * cols] component sizes, at the roots
+    unsigned long long* counts; // [2] or null
+};
+
+cudaError_t launch_speckles(const SpeckleParams& prm, int is_float, cudaStream_t stream);
+
 } // namespace bicos_b200

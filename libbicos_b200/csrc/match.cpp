@@ -5,6 +5,7 @@
 #include "../../include/BICOS/match.hpp"
 #include "../../include/BICOS/rectify.hpp"
 #include "../../include/BICOS/reproject.hpp"
+#include "../../include/BICOS/speckles.hpp"
 #include "../../include/bicos_b200.h"
 
 #include <cuda_runtime.h>
@@ -35,7 +36,7 @@ void cuda_check(cudaError_t err, const char* what) {
 // reference (which has no global mutable state), and repeated calls reuse their buffers.
 struct HandleCache {
     std::map<int, bicos_b200_handle> handles;
-    std::map<int, unsigned long long*> counts; // reproject_points: the four device counters
+    std::map<int, unsigned long long*> counts; // device counters: four of reproject_points, two of filter_speckles
     ~HandleCache() {
         for (auto& kv: counts) {
             cudaSetDevice(kv.first);
@@ -59,7 +60,7 @@ struct HandleCache {
 
 thread_local HandleCache t_handles;
 
-// the device counters of reproject_points on `device` (current)
+// the device counters of reproject_points and filter_speckles on `device` (current)
 unsigned long long* counts_buffer(int device) {
     auto it = t_handles.counts.find(device);
     if (it != t_handles.counts.end())
@@ -380,6 +381,26 @@ ReprojectCounts reproject_points(const Image& disparity, const std::array<double
     cuda_check(cudaMemcpyAsync(host, counts, sizeof host, cudaMemcpyDeviceToHost, s), "download counts");
     cuda_check(cudaStreamSynchronize(s), "cudaStreamSynchronize");
     return ReprojectCounts { (size_t)host[0], (size_t)host[1], (size_t)host[2], (size_t)host[3] };
+}
+
+void filter_speckles(Image& disparity, double new_value, int max_speckle_size, double max_diff, SpeckleCounts* counts, void* stream) {
+    if (disparity.empty() || (disparity.type() != IMG_16S && disparity.type() != IMG_32F))
+        throw Exception("speckle filtering needs a non-empty CV_16SC1 or CV_32FC1 disparity image");
+    const int device = device_of(disparity.data);
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    unsigned long long* dev_counts = counts ? counts_buffer(device) : nullptr;
+    const int rc = bicos_b200_filter_speckles(h, disparity.data, disparity.type(), disparity.step, disparity.rows, disparity.cols,
+                                              new_value, max_speckle_size, max_diff, dev_counts, stream);
+    if (rc != 0)
+        rethrow_last(rc);
+    if (!counts)
+        return;
+    unsigned long long host[2] = { 0, 0 };
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    cuda_check(cudaMemcpyAsync(host, dev_counts, sizeof host, cudaMemcpyDeviceToHost, s), "download counts");
+    cuda_check(cudaStreamSynchronize(s), "cudaStreamSynchronize");
+    *counts = SpeckleCounts { (size_t)host[0], (size_t)host[1] };
 }
 
 void match_sharded(
