@@ -152,6 +152,35 @@ int bicos_b200_search_range(bicos_b200_handle h, const uint32_t* desc0, const ui
                             uint32_t* fwd_last, uint32_t* rev_first, uint32_t* rev_last,
                             int min_disparity, int max_disparity, void* stream);
 
+/* ---- per-pixel disparity windows ----------------------------------------------------------
+ * A window map bounds the search pixel by pixel instead of with one range for the frame: e.g. a prior from the previous
+ * frame +- a margin, bounds from known geometry, or an empty window for every pixel outside a region of interest.
+ * min_disparity / max_disparity: device int16 images [rows][pitch_bytes], one pitch for both, even and at least
+ * cols * 2 (2-byte aligned pointers). Semantics:
+ *   left pixel (r, i) pairs with right column j iff min(r, i) <= i - j <= max(r, i), clipped to the row; min > max is
+ *   an empty window: the pixel is invalid (corrmap NaN) and nothing is searched or refined for it
+ *   the reverse search of the Consistency check from right column b runs over the left columns a with
+ *   min(r, a) <= a - b <= max(r, a): exactly the pairs the forward windows define (not necessarily contiguous)
+ *   ties as without windows (the first strict minimum; with no-dupes a second minimum invalidates); the refine is
+ *   unchanged, so a subpixel disparity may lie up to 1 px outside the window, as with a range
+ * Constant maps (m, M) give bit for bit the result of bicos_b200_config's range [m, M] (keys, disparity, corrmap);
+ * maps that cover the row, e.g. (-32768, 32767), give bit for bit the unranged match. Windows run on the integer-pipe
+ * engine: with BICOS_B200_SEARCH_TENSOR forced they fail with BICOS_B200_ERR_CUDA. */
+typedef struct {
+    const int16_t* min_disparity;
+    const int16_t* max_disparity;
+    size_t pitch_bytes;
+} bicos_b200_disparity_windows;
+
+/* Stage 2+4a over window maps, with the key contract of bicos_b200_search_range: the key arrays are filled by this
+ * call (the reverse ones prefilled here), fwd_last is required for every `flags` and always written (without
+ * FLAG_NODUPES as the mirror of fwd_first), and an empty window gets 0xFFFFFFFF in both forward arrays. To refine
+ * these keys, pass bicos_b200_refine a config with a range that does not cover the row (e.g. has_disparity_range = 1,
+ * [0, 0]): that turns on its first / last comparison, which rejects the empty windows. */
+int bicos_b200_search_windows(bicos_b200_handle h, const uint32_t* desc0, const uint32_t* desc1, int K, int rows, int cols,
+                              size_t desc_pitch_words, int flags, uint32_t* fwd_first, uint32_t* fwd_last, uint32_t* rev_first,
+                              uint32_t* rev_last, const bicos_b200_disparity_windows* windows, void* stream);
+
 /* Stage 4b+3, reference bicos<>() postfilter (bicos.hpp:95-110) + agree / agree_subpixel
  * (include/impl/cpu/agree.hpp:53-191) on the keys of bicos_b200_search. raw_disp_out
  * (optional, dense int16 [rows][cols]) receives the postfilter result before the NXC test. */
@@ -173,6 +202,27 @@ int bicos_b200_match(bicos_b200_handle h, const void* const* planes0, const void
                      int n, int rows, int cols, size_t pitch_bytes, int depth,
                      const bicos_b200_config* cfg, void* disparity, size_t disparity_pitch_bytes,
                      void* corrmap, size_t corrmap_pitch_bytes, void* stream);
+
+/* bicos_b200_match over window maps (see bicos_b200_disparity_windows): the same outputs and types, the search
+ * bounded per pixel. cfg->has_disparity_range must be 0 (windows and a range together are BICOS_B200_ERR_INVALID).
+ * Runs as one unit on `stream` (no row bands); like every match it first waits for the handle's previous work when
+ * that was enqueued on another stream. */
+int bicos_b200_match_windows(bicos_b200_handle h, const void* const* planes0, const void* const* planes1, int n, int rows,
+                             int cols, size_t pitch_bytes, int depth, const bicos_b200_config* cfg,
+                             const bicos_b200_disparity_windows* windows, void* disparity, size_t disparity_pitch_bytes,
+                             void* corrmap, size_t corrmap_pitch_bytes, void* stream);
+
+/* Window maps from a prior disparity, one launch. prior: device int16 (BICOS_B200_16S) or float32 (BICOS_B200_32F)
+ * [rows][prior_pitch_bytes], pitch a multiple of the element size. Per pixel:
+ *   invalid prior (int16 -32768; float32 NaN, -32768.0f or +-inf): (fallback_min, fallback_max), which may be empty
+ *   (min > max: the pixel is skipped) or cover the row
+ *   valid prior d: min = clamp(floor(d) - margin), max = clamp(ceil(d) + margin), clamp to [-32768, 32767], computed
+ *   exactly in double
+ * margin 0..32767; fallback bounds within int16; rows 1..65535, cols 1..32767; min_out / max_out as in
+ * bicos_b200_disparity_windows with windows_pitch_bytes. */
+int bicos_b200_windows_from_disparity(bicos_b200_handle h, const void* prior, int prior_type, size_t prior_pitch_bytes, int rows,
+                                      int cols, int margin, int fallback_min, int fallback_max, int16_t* min_out,
+                                      int16_t* max_out, size_t windows_pitch_bytes, void* stream);
 
 /* ---- rectification: raw camera stacks in ------------------------------------------------
  * The match expects rectified stacks (corresponding points on the same row). These entry points APPLY
@@ -371,7 +421,7 @@ int bicos_b200_set_search_engine(int engine);
 int bicos_b200_get_search_engine(void);
 
 /* Name of the kernel the calling thread's last search dispatched, e.g. "mma2<K=4,nodupes=0,ct=1,dirs=2>",
- * "mma1<...>", "popc<K=4,flags=2>" or, with a disparity range, "range<K=4,flags=2>"; "" before the first search. For tests and benchmarks that must know
+ * "mma1<...>", "popc<K=4,flags=2>", with a disparity range "range<K=4,flags=2>" and with window maps "windows<K=4,flags=2>"; "" before the first search. For tests and benchmarks that must know
  * which of the engine's kernels they exercised. The string is thread-local and valid until the next search. */
 const char* bicos_b200_last_search_kernel(void);
 

@@ -29,6 +29,7 @@ EXPORTS = (
     "bicos_b200_shared_alloc", "bicos_b200_shared_open", "bicos_b200_shared_close", "bicos_b200_shared_free",
     "bicos_b200_set_search_engine", "bicos_b200_get_search_engine", "bicos_b200_last_search_kernel",
     "bicos_b200_remap", "bicos_b200_match_rectified", "bicos_b200_reproject", "bicos_b200_filter_speckles",
+    "bicos_b200_search_windows", "bicos_b200_match_windows", "bicos_b200_windows_from_disparity",
 )
 SEARCH_ENGINES = {"auto": 0, "popc": 1, "tensor": 2}
 IPC_HANDLE_BYTES = 64
@@ -101,6 +102,12 @@ class CRectifyMaps(ctypes.Structure):
                 ("map_y1", ctypes.c_void_p), ("map_pitch_bytes", ctypes.c_size_t)]
 
 
+class CDisparityWindows(ctypes.Structure):
+    """bicos_b200_disparity_windows."""
+
+    _fields_ = [("min_disparity", ctypes.c_void_p), ("max_disparity", ctypes.c_void_p), ("pitch_bytes", ctypes.c_size_t)]
+
+
 @dataclass
 class RectifyMaps:
     """Rectification maps of both cameras for Handle.match_rectified: float32 CUDA tensors [rows, cols] with
@@ -162,6 +169,10 @@ def lib():
                                                  sz, vp]
         L.bicos_b200_reproject.argtypes = [vp, vp, i, sz, i, i, ctypes.POINTER(ctypes.c_double), i, vp, sz, vp, vp, vp, vp]
         L.bicos_b200_filter_speckles.argtypes = [vp, vp, i, sz, i, i, ctypes.c_double, i, ctypes.c_double, vp, vp]
+        winp = ctypes.POINTER(CDisparityWindows)
+        L.bicos_b200_search_windows.argtypes = [vp, vp, vp, i, i, i, sz, i, vp, vp, vp, vp, winp, vp]
+        L.bicos_b200_match_windows.argtypes = [vp, pp, pp, i, i, i, sz, i, cfgp, winp, vp, sz, vp, sz, vp]
+        L.bicos_b200_windows_from_disparity.argtypes = [vp, vp, i, sz, i, i, i, i, i, vp, vp, sz, vp]
         L.bicos_b200_stage_times.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_longlong)]
         _lib = L
     return _lib
@@ -266,7 +277,7 @@ class Handle:
                                           desc.data_ptr(), pitch_words, self._stream()))
         return desc, k
 
-    def search(self, desc0, desc1, k: int, cols: int, flags: int, top_bit_free=False, disparity_range=None):
+    def search(self, desc0, desc1, k: int, cols: int, flags: int, top_bit_free=False, disparity_range=None, windows=None):
         """Row-wise search on pitched descriptors -> (fwd_first, fwd_last, rev_first, rev_last).
 
         Each is a [rows, cols] int32 tensor holding uint32 keys cost << 16 | column (see
@@ -275,7 +286,9 @@ class Handle:
         transform() output), which lets the tensor-core engine use its column-term kernels; ``top_bit_free=2``: the
         top TWO bits are zero (BICOS_B200_FLAG_TOP2_BITS_FREE; also true for transform() output), which adds the
         one-pass consistency kernel. ``disparity_range`` = (min, max): only the pairs with min <= x_left - x_right <= max
-        (bicos_b200_search_range); fwd_last is then always returned, and refine() needs a Config with the same range."""
+        (bicos_b200_search_range); fwd_last is then always returned, and refine() needs a Config with the same range.
+        ``windows`` = (min, max) int16 CUDA tensors [rows, cols]: per-pixel bounds instead (bicos_b200_search_windows);
+        fwd_last is always returned, and refine() needs a Config with a range that does not cover the row, e.g. (0, 0)."""
         import torch
 
         rows, pitch_words = desc0.shape
@@ -285,12 +298,18 @@ class Handle:
             return torch.empty((rows, cols), dtype=torch.int32, device=dev) if needed else None
 
         fwdf = keys(True)
-        fwdl = keys(flags & FLAG_NODUPES or disparity_range is not None)
+        fwdl = keys(flags & FLAG_NODUPES or disparity_range is not None or windows is not None)
         revf = keys(flags & FLAG_CONSISTENCY)
         revl = keys(flags == (FLAG_NODUPES | FLAG_CONSISTENCY))
         ptr = [t.data_ptr() if t is not None else None for t in (fwdf, fwdl, revf, revl)]
         flags |= FLAG_TOP2_BITS_FREE if int(top_bit_free) >= 2 else FLAG_TOP_BIT_FREE if top_bit_free else 0
-        if disparity_range is None:
+        if windows is not None:
+            if disparity_range is not None:
+                raise BicosError("disparity windows and a disparity range exclude each other")
+            cw = self._windows_info(windows, rows, cols, dev)
+            _check(lib().bicos_b200_search_windows(self._h, desc0.data_ptr(), desc1.data_ptr(), k, rows, cols, pitch_words, flags,
+                                                   *ptr, ctypes.byref(cw), self._stream()))
+        elif disparity_range is None:
             _check(lib().bicos_b200_search(self._h, desc0.data_ptr(), desc1.data_ptr(), k, rows, cols, pitch_words, flags,
                                            *ptr, self._stream()))
         else:
@@ -399,6 +418,64 @@ class Handle:
             _check(lib().bicos_b200_match_rows(self._h, p0, p1, n, rows, cols, pitch, depth, ctypes.byref(ccfg),
                                                int(rows_range[0]), int(rows_range[1]), *args))
         return disp, corr
+
+    @staticmethod
+    def _windows_info(windows, rows: int, cols: int, device) -> CDisparityWindows:
+        """bicos_b200_disparity_windows of a (min, max) pair of int16 CUDA tensors [rows, cols] with one row stride."""
+        import torch
+
+        try:
+            wmin, wmax = windows
+        except (TypeError, ValueError):
+            raise BicosError("windows must be a (min_disparity, max_disparity) pair") from None
+        for m in (wmin, wmax):
+            if not isinstance(m, torch.Tensor) or m.dtype != torch.int16 or m.dim() != 2 or not m.is_cuda:
+                raise BicosError("disparity windows must be int16 CUDA tensors of shape [rows, cols]")
+            if m.device != device:
+                raise BicosError(f"a disparity window map lives on {m.device}, the stacks on {device}")
+            if tuple(m.shape) != (rows, cols) or m.stride(1) != 1:
+                raise BicosError(f"disparity window maps must have shape ({rows}, {cols}) with contiguous rows")
+        if wmin.stride(0) != wmax.stride(0):
+            raise BicosError("both disparity window maps must share one row stride")
+        return CDisparityWindows(wmin.data_ptr(), wmax.data_ptr(), wmin.stride(0) * 2)
+
+    def match_windows(self, stack0, stack1, windows, cfg: Config, out=None):
+        """match() with the search bounded per pixel (bicos_b200_match_windows): ``windows`` = (min, max) int16 CUDA
+        tensors [rows, cols]; left pixel (r, i) pairs with right column j iff min[r, i] <= i - j <= max[r, i], and
+        min > max makes the pixel invalid without searching it. ``cfg.disparity_range`` must be None.
+        ``out`` = (disparity, corrmap) tensors to reuse."""
+        p0, n, rows, cols, pitch, depth = self._stack_info(stack0)
+        p1, n1, rows1, cols1, pitch1, depth1 = self._stack_info(stack1)
+        if (n1, rows1, cols1, pitch1, depth1) != (n, rows, cols, pitch, depth):
+            raise BicosError("stack0 and stack1 differ")
+        cw = self._windows_info(windows, rows, cols, stack0.device)
+        if out is None:
+            ccfg, disp, corr = self._outputs(cfg, rows, cols, stack0.device)
+        else:
+            ccfg = cfg.to_c()
+            disp, corr = self._check_out(ccfg, out, rows, cols, stack0.device)
+        _check(lib().bicos_b200_match_windows(
+            self._h, p0, p1, n, rows, cols, pitch, depth, ctypes.byref(ccfg), ctypes.byref(cw), disp.data_ptr(),
+            disp.stride(0) * disp.element_size(), corr.data_ptr() if corr is not None else None,
+            corr.stride(0) * corr.element_size() if corr is not None else 0, self._stream()))
+        return disp, corr
+
+    def windows_from_disparity(self, prior, margin: int, fallback=None, out=None):
+        """Window maps from a prior disparity (bicos_b200_windows_from_disparity): [rows, cols] int16 / float32 CUDA
+        tensor -> (min, max) int16 tensors. A valid prior d gives [floor(d) - margin, ceil(d) + margin] clamped to int16;
+        an invalid one (-32768, NaN, -32768.0 or +-inf) gives ``fallback`` = (min, max), None = the whole row.
+        ``out`` = a (min, max) pair of int16 tensors [rows, cols] with one row stride to fill."""
+        import torch
+
+        code, rows, cols, pitch = self._disparity_info(prior)
+        fb = (-32768, 32767) if fallback is None else (int(fallback[0]), int(fallback[1]))
+        if out is None:
+            out = (torch.empty((rows, cols), dtype=torch.int16, device=prior.device),
+                   torch.empty((rows, cols), dtype=torch.int16, device=prior.device))
+        cw = self._windows_info(out, rows, cols, prior.device)
+        _check(lib().bicos_b200_windows_from_disparity(self._h, prior.data_ptr(), code, pitch, rows, cols, int(margin), fb[0], fb[1],
+                                                       cw.min_disparity, cw.max_disparity, cw.pitch_bytes, self._stream()))
+        return out
 
     @staticmethod
     def _map_info(maps, device):

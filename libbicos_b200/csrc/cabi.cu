@@ -486,7 +486,8 @@ int do_refine(
     size_t disparity_pitch,
     void* corrmap,
     size_t corrmap_pitch,
-    cudaStream_t stream
+    cudaStream_t stream,
+    bool windowed = false
 ) {
     RefineParams prm {};
     prm.n = n;
@@ -514,8 +515,8 @@ int do_refine(
         prm.xs = static_cast<const float*>(h->xs.ptr);
     }
     int dmin = 0, dmax = 0;
-    // ranged keys: the first / last comparison also rejects the empty windows (launch_search_range)
-    prm.nodupes_forward = (search_flags(cfg) & FLAG_NODUPES) != 0 || cfg_range(cfg, cols, &dmin, &dmax);
+    // ranged and windowed keys: the first / last comparison also rejects the empty windows (launch_search_range)
+    prm.nodupes_forward = (search_flags(cfg) & FLAG_NODUPES) != 0 || cfg_range(cfg, cols, &dmin, &dmax) || windowed;
     prm.fwd_first = fwd_first;
     prm.fwd_last = fwd_last;
     prm.rev_first = rev_first;
@@ -533,6 +534,7 @@ int do_refine(
 // One unit of work of the path: rows [row_begin, row_end) of one stereo stack, with the output rows it writes.
 struct Unit {
     PlaneTable t0, t1; // plane pointers already advanced to row_begin
+    int row_begin = 0;
     int nrows = 0;
     char* disp_rows = nullptr;
     char* corr_rows = nullptr;
@@ -540,8 +542,11 @@ struct Unit {
 
 struct MatchShape {
     int n, cols, K, depth, flags;
-    bool ranged; // a disparity range that excludes some pairs: the windowed search, [dmin, dmax] clipped
+    bool ranged; // a disparity range that excludes some pairs, or window maps: the windowed search, [dmin, dmax] clipped
     int dmin, dmax;
+    const int16_t* wmin; // window maps (bicos_b200_match_windows), [rows][wpitch elements] from the match's row 0; or null
+    const int16_t* wmax;
+    size_t wpitch;
     size_t pitch_bytes, disparity_pitch, corrmap_pitch;
     const bicos_b200_config* cfg;
 };
@@ -552,6 +557,7 @@ int make_unit(Unit& u, const void* const* planes0, const void* const* planes1, c
         return rc;
     if (int rc = fill_table(u.t1, planes1, sh.n, (size_t)row_begin * sh.pitch_bytes))
         return rc;
+    u.row_begin = row_begin;
     u.nrows = row_end - row_begin;
     u.disp_rows = static_cast<char*>(disparity) + (size_t)row_begin * sh.disparity_pitch;
     u.corr_rows = corrmap ? static_cast<char*>(corrmap) + (size_t)row_begin * sh.corrmap_pitch : nullptr;
@@ -580,8 +586,14 @@ int enqueue_search_stage(bicos_b200_handle h, const Unit& u, const MatchShape& s
     if (sh.ranged) {
         if (sh.flags & FLAG_CONSISTENCY) // reverse minima merge across CTAs with atomicMin; the forward keys are stored
             CU(cudaMemsetAsync(ka.rev_first, 0xFF, px * sizeof(uint32_t) * ((sh.flags & FLAG_NODUPES) ? 2 : 1), stream));
-        CU(launch_search_range(d0, d1, sh.K, u.nrows, sh.cols, dpw, sh.flags, sh.dmin, sh.dmax, ka.fwd_first, ka.fwd_last, ka.rev_first,
-                               ka.rev_last, stream));
+        if (sh.wmin) {
+            const size_t w0 = (size_t)u.row_begin * sh.wpitch;
+            CU(launch_search_windows(d0, d1, sh.K, u.nrows, sh.cols, dpw, sh.flags, sh.wmin + w0, sh.wmax + w0, sh.wpitch, ka.fwd_first,
+                                     ka.fwd_last, ka.rev_first, ka.rev_last, stream));
+        } else {
+            CU(launch_search_range(d0, d1, sh.K, u.nrows, sh.cols, dpw, sh.flags, sh.dmin, sh.dmax, ka.fwd_first, ka.fwd_last,
+                                   ka.rev_first, ka.rev_last, stream));
+        }
         h->launches += 1;
         return timer.end();
     }
@@ -599,7 +611,7 @@ int enqueue_refine_stage(bicos_b200_handle h, const Unit& u, const MatchShape& s
     StageTimer timer(h, 2, stream);
     KeyArrays ka = split_keys(keys, (size_t)u.nrows * sh.cols, sh.flags, sh.ranged);
     if (int rc = do_refine(h, u.t0, u.t1, sh.n, u.nrows, sh.cols, sh.pitch_bytes, sh.depth, sh.cfg, ka.fwd_first, ka.fwd_last, ka.rev_first,
-                           ka.rev_last, nullptr, u.disp_rows, sh.disparity_pitch, u.corr_rows, sh.corrmap_pitch, stream))
+                           ka.rev_last, nullptr, u.disp_rows, sh.disparity_pitch, u.corr_rows, sh.corrmap_pitch, stream, sh.wmin != nullptr))
         return rc;
     return timer.end();
 }
@@ -658,6 +670,17 @@ int leave_workspace(bicos_b200_handle h, cudaStream_t stream) {
     return 0;
 }
 
+// window maps for rows of `cols` pixels (bicos_b200_disparity_windows)
+int validate_windows(const bicos_b200_disparity_windows* w, int cols) {
+    if (!w || !w->min_disparity || !w->max_disparity)
+        return fail(BICOS_B200_ERR_INVALID, "disparity windows: a map is null");
+    if (w->pitch_bytes % 2 != 0 || w->pitch_bytes < (size_t)cols * 2 || reinterpret_cast<uintptr_t>(w->min_disparity) % 2 != 0 ||
+        reinterpret_cast<uintptr_t>(w->max_disparity) % 2 != 0)
+        return fail(BICOS_B200_ERR_INVALID, "disparity windows: pitch %zu must be even and at least cols * 2 = %d, maps 2-byte aligned",
+                    w->pitch_bytes, cols * 2);
+    return 0;
+}
+
 int do_match(
     bicos_b200_handle h,
     const void* const* planes0,
@@ -674,11 +697,24 @@ int do_match(
     size_t disparity_pitch,
     void* corrmap,
     size_t corrmap_pitch,
-    cudaStream_t stream
+    cudaStream_t stream,
+    const bicos_b200_disparity_windows* windows = nullptr
 ) {
     MatchShape sh {};
     if (int rc = validate_match(planes0, planes1, n, rows, cols, pitch_bytes, depth, cfg, disparity, sh))
         return rc;
+    if (windows) {
+        if (cfg->has_disparity_range)
+            return fail(BICOS_B200_ERR_INVALID, "disparity windows and a disparity range exclude each other");
+        if (int rc = validate_windows(windows, cols))
+            return rc;
+        if (int rc = check_range_engine())
+            return rc;
+        sh.ranged = true;
+        sh.wmin = windows->min_disparity;
+        sh.wmax = windows->max_disparity;
+        sh.wpitch = windows->pitch_bytes / 2;
+    }
     if (row_begin < 0 || row_end > rows || row_begin >= row_end)
         return fail(BICOS_B200_ERR_INVALID, "bad row range [%d, %d) of %d", row_begin, row_end, rows);
     sh.disparity_pitch = disparity_pitch;
@@ -943,6 +979,40 @@ int bicos_b200_search_range(bicos_b200_handle h, const uint32_t* desc0, const ui
     return 0;
 }
 
+int bicos_b200_search_windows(bicos_b200_handle h, const uint32_t* desc0, const uint32_t* desc1, int K, int rows, int cols,
+                              size_t desc_pitch_words, int flags, uint32_t* fwd_first, uint32_t* fwd_last, uint32_t* rev_first,
+                              uint32_t* rev_last, const bicos_b200_disparity_windows* windows, void* stream) {
+    if (!h || !desc0 || !desc1 || !fwd_first || !fwd_last)
+        return fail(BICOS_B200_ERR_INVALID, "null argument (a windowed search always needs fwd_last)");
+    if (K != 1 && K != 2 && K != 4 && K != 8 && K != 12 && K != 16)
+        return fail(BICOS_B200_ERR_INVALID, "K must be 1, 2, 4 or 8 (12 or 16 for wide descriptors)");
+    if (flags < 0 || flags > 15)
+        return fail(BICOS_B200_ERR_INVALID, "bad flags");
+    flags &= 3; // the top-bit promises only matter to the tensor-core engine
+    if (rows <= 0 || rows > 65535 || cols <= 0 || cols > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "bad image size");
+    if ((flags & FLAG_CONSISTENCY) && (!rev_first || ((flags & FLAG_NODUPES) && !rev_last)))
+        return fail(BICOS_B200_ERR_INVALID, "consistency search needs rev_first (and rev_last with no_dupes)");
+    if (desc_pitch_words < (size_t)cols * K || (desc_pitch_words % 4) != 0)
+        return fail(BICOS_B200_ERR_INVALID, "descriptor rows must be 16-byte aligned and hold cols*K words");
+    if (int rc = validate_windows(windows, cols))
+        return rc;
+    if (int rc = check_range_engine())
+        return rc;
+    DeviceGuard g(h->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const size_t bytes = (size_t)rows * cols * sizeof(uint32_t);
+    if (flags & FLAG_CONSISTENCY) {
+        CU(cudaMemsetAsync(rev_first, 0xFF, bytes, s));
+        if (flags & FLAG_NODUPES)
+            CU(cudaMemsetAsync(rev_last, 0xFF, bytes, s));
+    }
+    CU(launch_search_windows(desc0, desc1, K, rows, cols, desc_pitch_words, flags, windows->min_disparity, windows->max_disparity,
+                             windows->pitch_bytes / 2, fwd_first, fwd_last, rev_first, rev_last, s));
+    h->launches += 1;
+    return 0;
+}
+
 int bicos_b200_refine(bicos_b200_handle h, const void* const* planes0, const void* const* planes1,
                       int n, int rows, int cols, size_t pitch_bytes, int depth,
                       const bicos_b200_config* cfg, const uint32_t* fwd_first, const uint32_t* fwd_last,
@@ -1015,6 +1085,58 @@ int bicos_b200_match(bicos_b200_handle h, const void* const* planes0, const void
     DeviceGuard g(h->device);
     return match_banded_or_whole(h, planes0, planes1, n, rows, cols, pitch_bytes, depth, cfg, disparity,
                                  disparity_pitch_bytes, corrmap, corrmap_pitch_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int bicos_b200_match_windows(bicos_b200_handle h, const void* const* planes0, const void* const* planes1, int n, int rows,
+                             int cols, size_t pitch_bytes, int depth, const bicos_b200_config* cfg,
+                             const bicos_b200_disparity_windows* windows, void* disparity, size_t disparity_pitch_bytes,
+                             void* corrmap, size_t corrmap_pitch_bytes, void* stream) {
+    if (!h)
+        return fail(BICOS_B200_ERR_INVALID, "null handle");
+    if (!windows)
+        return fail(BICOS_B200_ERR_INVALID, "disparity windows are null");
+    DeviceGuard g(h->device);
+    return do_match(h, planes0, planes1, n, rows, cols, pitch_bytes, depth, cfg, 0, rows, disparity, disparity_pitch_bytes, corrmap,
+                    corrmap_pitch_bytes, static_cast<cudaStream_t>(stream), windows);
+}
+
+int bicos_b200_windows_from_disparity(bicos_b200_handle h, const void* prior, int prior_type, size_t prior_pitch_bytes, int rows,
+                                      int cols, int margin, int fallback_min, int fallback_max, int16_t* min_out,
+                                      int16_t* max_out, size_t windows_pitch_bytes, void* stream) {
+    if (!h || !prior || !min_out || !max_out)
+        return fail(BICOS_B200_ERR_INVALID, "null argument");
+    if (prior_type != BICOS_B200_16S && prior_type != BICOS_B200_32F)
+        return fail(BICOS_B200_ERR_INVALID, "bad prior type %d: only int16 (CV_16SC1) and float32 (CV_32FC1)", prior_type);
+    if (rows < 1 || cols < 1 || rows > 65535 || cols > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "prior of %d x %d: rows 1 to 65535, cols 1 to 32767", rows, cols);
+    const size_t es = prior_type == BICOS_B200_16S ? 2 : 4;
+    if (prior_pitch_bytes < (size_t)cols * es || prior_pitch_bytes % es != 0 || reinterpret_cast<uintptr_t>(prior) % es != 0)
+        return fail(BICOS_B200_ERR_INVALID, "prior rows must be aligned to and hold cols elements");
+    if (margin < 0 || margin > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "margin %d outside 0..32767", margin);
+    if (fallback_min < -32768 || fallback_min > 32767 || fallback_max < -32768 || fallback_max > 32767)
+        return fail(BICOS_B200_ERR_INVALID, "fallback window [%d, %d] outside int16", fallback_min, fallback_max);
+    const bicos_b200_disparity_windows w { min_out, max_out, windows_pitch_bytes };
+    if (int rc = validate_windows(&w, cols))
+        return rc;
+    DeviceGuard g(h->device);
+    WindowsParams prm {};
+    prm.prior = prior;
+    prm.prior_pitch = prior_pitch_bytes;
+    prm.rows = rows;
+    prm.cols = cols;
+    prm.margin = margin;
+    prm.fallback_min = fallback_min;
+    prm.fallback_max = fallback_max;
+    prm.min_out = min_out;
+    prm.max_out = max_out;
+    prm.out_pitch = windows_pitch_bytes / 2;
+    {
+        Range nvtx("bicos_b200::windows_from_disparity");
+        CU(launch_windows_from_disparity(prm, prior_type == BICOS_B200_32F, static_cast<cudaStream_t>(stream)));
+        h->launches += 1;
+    }
+    return 0;
 }
 
 // checks shared by bicos_b200_remap and bicos_b200_match_rectified

@@ -1,12 +1,13 @@
 // bicos-cli on the B200 path: same options, defaults and outputs as the reference CLI
 // (reference src/cli.cpp:55-253), without its dependencies (cxxopts, fmt, OpenCV): the argument
 // parser and the image I/O (imageio.cpp) are self-contained, the matching is BICOS::match from
-// include/BICOS/match.hpp, the point cloud of -q is BICOS::reproject_points from include/BICOS/reproject.hpp and
-// --speckles is BICOS::filter_speckles from include/BICOS/speckles.hpp.
+// include/BICOS/match.hpp, the point cloud of -q is BICOS::reproject_points from include/BICOS/reproject.hpp,
+// --speckles is BICOS::filter_speckles from include/BICOS/speckles.hpp and --disparity-prior is
+// BICOS::windows_from_disparity + BICOS::match_windows from include/BICOS/windows.hpp.
 //
 //   bicos-cli folder0 [folder1] [-t thr] [-v var] [-s step] [-o out.png] [-n N] [-q Q.yaml]
 //             [--allow-negative-z] [-m lr-maxdiff] [--double] [--limited] [--corrmap] [--no-dupes] [--wide-descriptors]
-//             [--disparity-range MIN:MAX] [--speckles SIZE:DIFF]
+//             [--disparity-range MIN:MAX] [--disparity-prior FILE:MARGIN] [--speckles SIZE:DIFF]
 //
 // Differences, on purpose: --allow-negative-z is honoured (the reference reads a non-existent
 // "allow-behind" option, cli.cpp:231); integer-mode disparities with a threshold are float32
@@ -15,6 +16,7 @@
 #include <BICOS/match.hpp>
 #include <BICOS/reproject.hpp>
 #include <BICOS/speckles.hpp>
+#include <BICOS/windows.hpp>
 
 #include "imageio.hpp"
 
@@ -67,6 +69,7 @@ const Option OPTIONS[] = {
     { "no-dupes", 0, false, "Default BICOS variant when --lr-maxdiff is not specified. Can be set together with --lr-maxdiff to activate both." },
     { "wide-descriptors", 0, false, "Extension: accept 17..23 images without --limited (384 / 512-bit descriptors; the reference stops at 16)." },
     { "disparity-range", 0, true, "Extension: search only disparities MIN..MAX (inclusive, may be negative), e.g. 0:127. (default: the whole row)" },
+    { "disparity-prior", 0, true, "Extension: search only within MARGIN px of the disparity in FILE, an int16 or float32 .tiff this tool wrote for the same image size, e.g. last.tiff:4. Pixels without a valid prior search --disparity-range, else the whole row. (default: off)" },
     { "speckles", 0, true, "Extension: after the match, mark connected blobs of at most SIZE pixels whose neighbours differ by at most DIFF as invalid, e.g. 100:1. (default: off)" },
     { "help", 'h', false, "Display this message." },
 };
@@ -345,6 +348,22 @@ int run(int argc, char const* const* argv) {
     }
     if (args.has("lr-maxdiff"))
         c.variant = Variant::Consistency { (int)to_uint(args, "lr-maxdiff"), args.has("no-dupes") };
+    std::optional<std::pair<std::string, int>> prior;
+    if (args.has("disparity-prior")) {
+        const std::string& v = args.get("disparity-prior");
+        const size_t colon = v.rfind(':');
+        size_t used = 0;
+        int margin = -1;
+        try {
+            if (colon != std::string::npos && colon > 0)
+                margin = std::stoi(v.substr(colon + 1), &used);
+        } catch (const std::exception&) {
+            used = 0;
+        }
+        if (used == 0 || used != v.size() - colon - 1 || margin < 0 || margin > 32767)
+            throw std::invalid_argument("Option 'disparity-prior' expects FILE:MARGIN with MARGIN in 0..32767, got '" + v + "'");
+        prior = std::make_pair(v.substr(0, colon), margin);
+    }
     std::optional<std::pair<int, double>> speckles;
     if (args.has("speckles")) {
         const std::string& v = args.get("speckles");
@@ -370,9 +389,23 @@ int run(int argc, char const* const* argv) {
     std::printf("Latency:\t %gms (upload)\t", ms_since(tick));
     std::fflush(stdout);
 
+    DisparityWindows windows;
+    if (prior) {
+        const DisparityImage p = read_disparity_tiff(prior->first);
+        if (p.rows != lstack.front().rows || p.cols != lstack.front().cols)
+            throw std::invalid_argument("disparity prior " + prior->first + " is " + std::to_string(p.cols) + "x" + std::to_string(p.rows) +
+                                        ", the images " + std::to_string(lstack.front().cols) + "x" + std::to_string(lstack.front().rows));
+        const Image prior_gpu(HostImage(p.rows, p.cols, p.type, const_cast<uint8_t*>(p.data.data())));
+        windows_from_disparity(prior_gpu, prior->second, c.disparity_range, windows);
+        c.disparity_range = std::nullopt; // now the fallback of the windows
+    }
+
     Image disp_gpu, corr_gpu;
     tick = std::chrono::high_resolution_clock::now();
-    BICOS::match(lstack, rstack, disp_gpu, c, need_corrmap ? &corr_gpu : nullptr);
+    if (prior)
+        match_windows(lstack, rstack, windows, disp_gpu, c, need_corrmap ? &corr_gpu : nullptr);
+    else
+        BICOS::match(lstack, rstack, disp_gpu, c, need_corrmap ? &corr_gpu : nullptr);
     SpeckleCounts removed {};
     if (speckles) {
         // speckles become the type's invalid marker, so the masking below applies unchanged: int16 -32768; float32 NaN

@@ -460,6 +460,65 @@ GrayImage read_tiff(const std::vector<uint8_t>& file, const std::string& path, b
     return img;
 }
 
+// the disparity TIFFs write_tiff produces, read back as a prior (bicos-cli --disparity-prior): one channel,
+// uncompressed strips, int16 (SampleFormat 2) or float32 (SampleFormat 3), either byte order
+DisparityImage read_disparity_tiff(const std::vector<uint8_t>& file, const std::string& path) {
+    TiffReader t { file, path };
+    if (file.size() < 8 || !((file[0] == 'I' && file[1] == 'I') || (file[0] == 'M' && file[1] == 'M')))
+        t.fail("not a TIFF file");
+    t.big = file[0] == 'M';
+    if (t.u16(2) != 42)
+        t.fail("not a TIFF file (BigTIFF is not supported)");
+    const size_t ifd = t.u32(4);
+    const int entries = t.u16(ifd);
+    uint32_t width = 0, height = 0, bits = 1, compression = 1, spp = 1, rows_per_strip = 0xFFFFFFFFu, sample_format = 1;
+    std::vector<uint32_t> offsets, counts;
+    for (int e = 0; e < entries; ++e) {
+        const size_t at = ifd + 2 + 12 * (size_t)e;
+        const std::vector<uint32_t> v = t.values(at);
+        if (v.empty())
+            t.fail("empty TIFF tag");
+        switch (t.u16(at)) {
+            case 256: width = v[0]; break;
+            case 257: height = v[0]; break;
+            case 258: bits = v[0]; break;
+            case 259: compression = v[0]; break;
+            case 273: offsets = v; break;
+            case 277: spp = v[0]; break;
+            case 278: rows_per_strip = v[0]; break;
+            case 279: counts = v; break;
+            case 339: sample_format = v[0]; break;
+            case 322: case 323: case 324: case 325: t.fail("tiled TIFF is not supported");
+            default: break;
+        }
+    }
+    if (width == 0 || height == 0 || width > 32767u || height > 65535u)
+        t.fail("TIFF without a size, or larger than 32767 x 65535");
+    if (spp != 1 || compression != 1 || !((bits == 16 && sample_format == 2) || (bits == 32 && sample_format == 3)))
+        t.fail("a disparity TIFF is one uncompressed channel of int16 or float32");
+    if (offsets.empty() || offsets.size() != counts.size() || rows_per_strip == 0)
+        t.fail("TIFF without strips");
+    rows_per_strip = std::min(rows_per_strip, height);
+    if ((size_t)(height + rows_per_strip - 1) / rows_per_strip != offsets.size())
+        t.fail("TIFF strip count does not match its height");
+    const size_t bps = bits / 8, row_bytes = (size_t)width * bps;
+    DisparityImage img;
+    img.rows = (int)height;
+    img.cols = (int)width;
+    img.type = bits == 16 ? 3 : 5;
+    img.data.reserve(row_bytes * height);
+    for (size_t sidx = 0; sidx < offsets.size(); ++sidx) {
+        const size_t expect = std::min<size_t>(rows_per_strip, height - sidx * rows_per_strip) * row_bytes;
+        if ((size_t)offsets[sidx] + counts[sidx] > file.size() || counts[sidx] < expect)
+            t.fail("short TIFF strip");
+        img.data.insert(img.data.end(), &file[offsets[sidx]], &file[offsets[sidx]] + expect);
+    }
+    if (t.big) // to the host's (little-endian) order
+        for (size_t i = 0; i < img.data.size(); i += bps)
+            std::reverse(&img.data[i], &img.data[i] + bps);
+    return img;
+}
+
 void put_be32(std::vector<uint8_t>& v, uint32_t x) {
     v.push_back(x >> 24);
     v.push_back(x >> 16);
@@ -485,6 +544,10 @@ GrayImage read_image(const std::string& path, bool& was_colour) {
     if (file.size() >= 8 && ((file[0] == 'I' && file[1] == 'I') || (file[0] == 'M' && file[1] == 'M')))
         return read_tiff(file, path, was_colour);
     return read_png(file, path, was_colour);
+}
+
+DisparityImage read_disparity_tiff(const std::string& path) {
+    return read_disparity_tiff(slurp(path), path);
 }
 
 #include "colormaps.inc"

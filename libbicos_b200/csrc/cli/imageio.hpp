@@ -5,7 +5,7 @@
 //   reference src/cli.cpp:228-250 (Q matrix, reprojection)
 // Readers: PNG (8/16-bit gray, gray+alpha, RGB, RGBA, palette; non-interlaced), binary PGM
 // (P5, 8/16 bit) and strip TIFF (8/16-bit gray or RGB[A]; uncompressed, LZW, Deflate, PackBits; both
-// byte orders) -- the formats multi-shot camera rigs dump. Writers: 8-bit RGB PNG, single-strip uncompressed TIFF (int16 / float32 /
+// byte orders) -- the formats multi-shot camera rigs dump -- and the int16 / float32 disparity TIFFs of write_tiff. Writers: 8-bit RGB PNG, single-strip uncompressed TIFF (int16 / float32 /
 // float64), ASCII .xyz. zlib is the only library used.
 #pragma once
 
@@ -30,6 +30,16 @@ enum class Colormap { TURBO, VIRIDIS };
 void colormap_lut(Colormap map, uint8_t lut[256][3]);
 
 void write_png_rgb(const std::string& path, int rows, int cols, const std::vector<uint8_t>& rgb);
+
+struct DisparityImage {
+    int rows = 0, cols = 0;
+    int type = 3; // 3 = int16, 5 = float32
+    std::vector<uint8_t> data; // dense rows, native-endian
+};
+
+// the single-channel disparity TIFFs write_tiff writes: uncompressed strips of int16 (SampleFormat 2, 16 bits) or
+// float32 (SampleFormat 3, 32 bits); anything else throws std::runtime_error with the file name
+DisparityImage read_disparity_tiff(const std::string& path);
 
 // sample_format: 1 = unsigned int, 2 = signed int, 3 = IEEE float
 void write_tiff(const std::string& path, int rows, int cols, int bits, int sample_format, const void* data);

@@ -174,6 +174,27 @@ cudaError_t launch_search_range(
     uint32_t* rev_last,
     cudaStream_t stream
 );
+// The same kernel over per-pixel windows (bicos_b200_search_windows): left pixel (r, i) pairs with right column j iff
+// wmin[r][i] <= i - j <= wmax[r][i], wmin / wmax int16 [rows][wpitch elements], advanced to the first row. Same key
+// contract as launch_search_range (fwd_last always written, rev_* pre-filled by the caller, KEY_NONE in both forward
+// arrays for an empty window, refine with nodupes_forward = 1).
+cudaError_t launch_search_windows(
+    const uint32_t* desc0,
+    const uint32_t* desc1,
+    int K,
+    int rows,
+    int cols,
+    size_t desc_pitch_words,
+    int flags,
+    const int16_t* wmin,
+    const int16_t* wmax,
+    size_t wpitch,
+    uint32_t* fwd_first,
+    uint32_t* fwd_last,
+    uint32_t* rev_first,
+    uint32_t* rev_last,
+    cudaStream_t stream
+);
 // Clips [*dmin, *dmax] to [-cols, cols] in place (i - j lies in [-(cols-1), cols-1], so the pairs stay the
 // same); false when the range covers every pair of the row, i.e. means exactly "no range" and the full-row
 // search applies.
@@ -254,5 +275,19 @@ struct SpeckleParams {
 };
 
 cudaError_t launch_speckles(const SpeckleParams& prm, int is_float, cudaStream_t stream);
+
+// disparity windows from a prior (windows.cu), with the semantics bicos_b200_windows_from_disparity states; one launch
+struct WindowsParams {
+    const void* prior; // int16 or float32 [rows][prior_pitch bytes]
+    size_t prior_pitch;
+    int rows, cols; // 1 .. 32767 columns, 1 .. 65535 rows
+    int margin; // 0 .. 32767
+    int fallback_min, fallback_max; // int16 values, for an invalid prior
+    int16_t* min_out; // [rows][out_pitch elements]
+    int16_t* max_out;
+    size_t out_pitch;
+};
+
+cudaError_t launch_windows_from_disparity(const WindowsParams& p, int is_float, cudaStream_t stream);
 
 } // namespace bicos_b200

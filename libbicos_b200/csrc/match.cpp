@@ -6,6 +6,7 @@
 #include "../../include/BICOS/rectify.hpp"
 #include "../../include/BICOS/reproject.hpp"
 #include "../../include/BICOS/speckles.hpp"
+#include "../../include/BICOS/windows.hpp"
 #include "../../include/bicos_b200.h"
 
 #include <cuda_runtime.h>
@@ -331,6 +332,67 @@ void match_rectified(
     const int rc = bicos_b200_match_rectified(h, v0.planes.data(), v1.planes.data(), (int)stack0.size(), v0.rows, v0.cols, v0.step,
                                               v0.depth, &m, rows, cols, &c, disparity.data, disparity.step,
                                               want_corr ? corrmap->data : nullptr, want_corr ? corrmap->step : 0, stream);
+    if (rc != 0)
+        rethrow_last(rc);
+}
+
+namespace {
+
+// a window pair of the disparity's size: CV_16SC1 device images of one pitch
+bicos_b200_disparity_windows windows_of(const DisparityWindows& w, int rows, int cols) {
+    for (const Image* m: { &w.min, &w.max })
+        if (m->empty() || m->type() != IMG_16S || m->rows != rows || m->cols != cols || m->step != w.min.step)
+            throw Exception("disparity windows must be non-empty CV_16SC1 images of the stacks' size and one pitch");
+    return bicos_b200_disparity_windows { reinterpret_cast<const int16_t*>(w.min.data), reinterpret_cast<const int16_t*>(w.max.data),
+                                          w.min.step };
+}
+
+} // namespace
+
+void match_windows(
+    const std::vector<Image>& stack0,
+    const std::vector<Image>& stack1,
+    const DisparityWindows& windows,
+    Image& disparity,
+    Config cfg,
+    Image* corrmap,
+    void* stream
+) {
+    const StackView v0 = view_of(stack0, "stack0");
+    const StackView v1 = view_of(stack1, "stack1");
+    if (stack0.size() != stack1.size() || v0.rows != v1.rows || v0.cols != v1.cols || v0.depth != v1.depth || v0.step != v1.step)
+        throw Exception("stack0 and stack1 differ in length, size, type or pitch");
+    const bicos_b200_disparity_windows w = windows_of(windows, v0.rows, v0.cols);
+    const bicos_b200_config c = to_c_config(cfg);
+    const int device = device_of(v0.planes.front());
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    disparity.create(v0.rows, v0.cols, bicos_b200_disparity_type(&c));
+    const bool want_corr = corrmap && cfg.nxcorr_threshold.has_value();
+    if (want_corr)
+        corrmap->create(v0.rows, v0.cols, bicos_b200_corrmap_type(&c));
+    const int rc = bicos_b200_match_windows(h, v0.planes.data(), v1.planes.data(), (int)stack0.size(), v0.rows, v0.cols, v0.step,
+                                            v0.depth, &c, &w, disparity.data, disparity.step, want_corr ? corrmap->data : nullptr,
+                                            want_corr ? corrmap->step : 0, stream);
+    if (rc != 0)
+        rethrow_last(rc);
+}
+
+void windows_from_disparity(const Image& prior, int margin, std::optional<DisparityRange> fallback, DisparityWindows& windows,
+                            void* stream) {
+    if (prior.empty() || (prior.type() != IMG_16S && prior.type() != IMG_32F))
+        throw Exception("windows_from_disparity needs a non-empty CV_16SC1 or CV_32FC1 prior");
+    const int device = device_of(prior.data);
+    bicos_b200_handle h = t_handles.get(device);
+    DeviceScope scope(device);
+    windows.min.create(prior.rows, prior.cols, IMG_16S);
+    windows.max.create(prior.rows, prior.cols, IMG_16S);
+    if (windows.max.step != windows.min.step)
+        throw Exception("disparity windows differ in pitch");
+    const DisparityRange fb = fallback.value_or(DisparityRange { -32768, 32767 });
+    const int rc = bicos_b200_windows_from_disparity(h, prior.data, prior.type(), prior.step, prior.rows, prior.cols, margin, fb.min,
+                                                     fb.max, reinterpret_cast<int16_t*>(windows.min.data),
+                                                     reinterpret_cast<int16_t*>(windows.max.data), windows.min.step, stream);
     if (rc != 0)
         rethrow_last(rc);
 }

@@ -16,9 +16,17 @@
 // per CTA with REDUX + shared atomics, CTAs with global atomicMin into key arrays the caller has
 // filled with KEY_NONE. Every left pixel belongs to one CTA, so the forward keys are plain stores
 // and fwd_last is always written (the contract with the refine in kernels.cuh).
+//
+// Windows (MAPS, bicos_b200_search_windows): the bounds come per left pixel from two int16 maps instead of one range.
+// Each lane clips its own window to the row and walks the same masked test with its own lo and span; the warp walks the
+// union of its lanes' windows, unmasked over their intersection, and the CTA stages the union of its warps' windows.
+// A lane with an empty window, or past the end of the row, gets lo = WIN_EMPTY_LO and span 0: j - lo is negative for
+// every column j of the row, so the unsigned test fails everywhere.
 
 #include "kernels.cuh"
 #include "search_common.cuh"
+
+#include <climits>
 
 namespace bicos_b200 {
 namespace {
@@ -38,7 +46,12 @@ struct RangeArgs {
     uint32_t* fwd_last;
     uint32_t* rev_first;
     uint32_t* rev_last;
+    const int16_t* wmin; // MAPS: [rows][wpitch] per-pixel bounds of i - j, advanced to the unit's first row
+    const int16_t* wmax;
+    size_t wpitch; // elements
 };
+
+constexpr int WIN_EMPTY_LO = 0x40000000; // see the header comment: fails (uint32_t)(j - lo) <= 0 for every j of a row
 
 template<int K>
 __device__ __forceinline__ uint32_t make_key(uint32_t h, uint32_t col, const Weights w) {
@@ -105,7 +118,13 @@ __device__ __forceinline__ void walk(
     }
 }
 
-template<int K, int FLAGS>
+// MAPS: the first and the last column of each warp's union of windows
+__device__ __forceinline__ int* window_bounds() {
+    __shared__ int s_win[2 * (RT / 32)];
+    return s_win;
+}
+
+template<int K, int FLAGS, bool MAPS>
 __global__ void __launch_bounds__(RT) search_range_kernel(const RangeArgs p) {
     constexpr bool NODUPES = (FLAGS & FLAG_NODUPES) != 0;
     constexpr bool REVERSE = (FLAGS & FLAG_CONSISTENCY) != 0;
@@ -134,12 +153,45 @@ __global__ void __launch_bounds__(RT) search_range_kernel(const RangeArgs p) {
     // the warp's pixels [xw, xe] and window [wlo, whi]; interior [ilo, ihi]: every valid lane in range
     const int xw = x0 + (tid & ~31);
     const int xe = min(xw + 31, cols - 1);
-    const int wlo = max(0, xw - p.dmax), whi = min(cols - 1, xe - p.dmin);
-    const int ilo = xe - p.dmax, ihi = xw - p.dmin;
-    const uint32_t span = (uint32_t)(p.dmax - p.dmin);
+    int wlo = max(0, xw - p.dmax), whi = min(cols - 1, xe - p.dmin);
+    int ilo = xe - p.dmax, ihi = xw - p.dmin;
+    uint32_t span = (uint32_t)(p.dmax - p.dmin);
     // the CTA's window: the union of its warps' windows (they overlap or touch), start 16 B aligned
-    const int clo = max(0, x0 - p.dmax) & ~3;
-    const int chi = min(cols - 1, min(x0 + RT, cols) - 1 - p.dmin);
+    int clo = max(0, x0 - p.dmax) & ~3;
+    int chi = min(cols - 1, min(x0 + RT, cols) - 1 - p.dmin);
+    int lo = 0; // MAPS: this lane's first right column (the range passes i - dmax)
+    if constexpr (MAPS) {
+        int* const s_win = window_bounds();
+        // this lane's right columns [i - max, i - min], clipped to the row (int16 bounds: no overflow)
+        int a = cols, b = -1;
+        if (valid) {
+            const size_t at = (size_t)row * p.wpitch + i;
+            a = max(0, i - (int)p.wmax[at]);
+            b = min(cols - 1, i - (int)p.wmin[at]);
+        }
+        const bool empty = a > b; // also every lane past the end of the row
+        lo = empty ? WIN_EMPTY_LO : a;
+        span = empty ? 0u : (uint32_t)(b - a);
+        // union over all lanes; intersection over the lanes in the row (an empty one empties it): past-the-end lanes
+        // carry bit 31 in their reverse keys and store nothing, so they may run unmasked (search.cu)
+        wlo = __reduce_min_sync(0xFFFFFFFFu, empty ? INT_MAX : a);
+        whi = __reduce_max_sync(0xFFFFFFFFu, empty ? -1 : b);
+        ilo = __reduce_max_sync(0xFFFFFFFFu, !valid ? INT_MIN : empty ? INT_MAX : a);
+        ihi = __reduce_min_sync(0xFFFFFFFFu, !valid ? INT_MAX : empty ? -1 : b);
+        if (lane == 0) {
+            s_win[tid >> 5] = wlo;
+            s_win[(tid >> 5) + RT / 32] = whi;
+        }
+        __syncthreads();
+        clo = INT_MAX;
+        chi = -1;
+#pragma unroll
+        for (int w = 0; w < RT / 32; ++w) {
+            clo = min(clo, s_win[w]);
+            chi = max(chi, s_win[w + RT / 32]);
+        }
+        clo &= ~3; // every pixel of the CTA empty: clo = INT_MAX & ~3 > chi = -1 skips the staging
+    }
 
     for (int c0 = clo; c0 <= chi; c0 += p.chunk) {
         const int cnt = min(p.chunk, chi + 1 - c0);
@@ -159,13 +211,13 @@ __global__ void __launch_bounds__(RT) search_range_kernel(const RangeArgs p) {
         }
         __syncthreads();
 
-        if (xw < cols) { // warp-uniform
+        if (xw < cols) { // warp-uniform; an all-empty warp of a window map has wlo > whi and walks nothing
             const int a = max(wlo, c0), b = min(whi + 1, c0 + cnt);
             if (a < b) {
                 const int ia = min(max(ilo, a), b), ib = min(max(ihi + 1, ia), b);
-                walk<K, FLAGS, true>(s_right, c0, a, ia, l, i - p.dmax, span, icol, icol_rev, lane, wts, mf, ml, s_colf, s_coll);
-                walk<K, FLAGS, false>(s_right, c0, ia, ib, l, i - p.dmax, span, icol, icol_rev, lane, wts, mf, ml, s_colf, s_coll);
-                walk<K, FLAGS, true>(s_right, c0, ib, b, l, i - p.dmax, span, icol, icol_rev, lane, wts, mf, ml, s_colf, s_coll);
+                walk<K, FLAGS, true>(s_right, c0, a, ia, l, MAPS ? lo : i - p.dmax, span, icol, icol_rev, lane, wts, mf, ml, s_colf, s_coll);
+                walk<K, FLAGS, false>(s_right, c0, ia, ib, l, MAPS ? lo : i - p.dmax, span, icol, icol_rev, lane, wts, mf, ml, s_colf, s_coll);
+                walk<K, FLAGS, true>(s_right, c0, ib, b, l, MAPS ? lo : i - p.dmax, span, icol, icol_rev, lane, wts, mf, ml, s_colf, s_coll);
             }
         }
 
@@ -208,10 +260,10 @@ int range_smem_bytes(int K, int chunk, int flags) {
     return bytes;
 }
 
-template<int K, int FLAGS>
+template<int K, int FLAGS, bool MAPS>
 cudaError_t launch_one(const RangeArgs& p, int rows, cudaStream_t stream) {
     const int smem = range_smem_bytes(K, p.chunk, FLAGS);
-    auto kernel = search_range_kernel<K, FLAGS>;
+    auto kernel = search_range_kernel<K, FLAGS, MAPS>;
     cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (err != cudaSuccess)
         return err;
@@ -220,17 +272,39 @@ cudaError_t launch_one(const RangeArgs& p, int rows, cudaStream_t stream) {
     return cudaGetLastError();
 }
 
-template<int K>
+template<int K, bool MAPS>
 cudaError_t launch_k(const RangeArgs& p, int rows, int flags, cudaStream_t stream) {
     switch (flags) {
         case FLAG_NODUPES:
-            return launch_one<K, FLAG_NODUPES>(p, rows, stream);
+            return launch_one<K, FLAG_NODUPES, MAPS>(p, rows, stream);
         case FLAG_CONSISTENCY:
-            return launch_one<K, FLAG_CONSISTENCY>(p, rows, stream);
+            return launch_one<K, FLAG_CONSISTENCY, MAPS>(p, rows, stream);
         case FLAG_NODUPES | FLAG_CONSISTENCY:
-            return launch_one<K, FLAG_NODUPES | FLAG_CONSISTENCY>(p, rows, stream);
+            return launch_one<K, FLAG_NODUPES | FLAG_CONSISTENCY, MAPS>(p, rows, stream);
         case 0:
-            return launch_one<K, 0>(p, rows, stream);
+            return launch_one<K, 0, MAPS>(p, rows, stream);
+    }
+    return cudaErrorInvalidValue;
+}
+
+template<bool MAPS>
+cudaError_t launch_args(RangeArgs& p, int K, int rows, int flags, cudaStream_t stream) {
+    p.one = 1u;
+    p.two = 2u;
+    p.shl16 = 65536u;
+    switch (K) {
+        case 1:
+            return launch_k<1, MAPS>(p, rows, flags, stream);
+        case 2:
+            return launch_k<2, MAPS>(p, rows, flags, stream);
+        case 4:
+            return launch_k<4, MAPS>(p, rows, flags, stream);
+        case 8:
+            return launch_k<8, MAPS>(p, rows, flags, stream);
+        case 12:
+            return launch_k<12, MAPS>(p, rows, flags, stream);
+        case 16:
+            return launch_k<16, MAPS>(p, rows, flags, stream);
     }
     return cudaErrorInvalidValue;
 }
@@ -264,7 +338,7 @@ cudaError_t launch_search_range(
         return cudaErrorInvalidValue;
     disparity_range_clip(cols, &dmin, &dmax);
     note_search_kernel("range<K=%d,flags=%d>", K, flags);
-    RangeArgs p;
+    RangeArgs p {};
     p.desc0 = desc0;
     p.desc1 = desc1;
     p.cols = cols;
@@ -272,28 +346,50 @@ cudaError_t launch_search_range(
     p.dmin = dmin;
     p.dmax = dmax;
     p.chunk = range_chunk(K, dmin, dmax);
-    p.one = 1u;
-    p.two = 2u;
-    p.shl16 = 65536u;
     p.fwd_first = fwd_first;
     p.fwd_last = fwd_last;
     p.rev_first = rev_first;
     p.rev_last = rev_last;
-    switch (K) {
-        case 1:
-            return launch_k<1>(p, rows, flags, stream);
-        case 2:
-            return launch_k<2>(p, rows, flags, stream);
-        case 4:
-            return launch_k<4>(p, rows, flags, stream);
-        case 8:
-            return launch_k<8>(p, rows, flags, stream);
-        case 12:
-            return launch_k<12>(p, rows, flags, stream);
-        case 16:
-            return launch_k<16>(p, rows, flags, stream);
-    }
-    return cudaErrorInvalidValue;
+    return launch_args<false>(p, K, rows, flags, stream);
+}
+
+cudaError_t launch_search_windows(
+    const uint32_t* desc0,
+    const uint32_t* desc1,
+    int K,
+    int rows,
+    int cols,
+    size_t desc_pitch_words,
+    int flags,
+    const int16_t* wmin,
+    const int16_t* wmax,
+    size_t wpitch,
+    uint32_t* fwd_first,
+    uint32_t* fwd_last,
+    uint32_t* rev_first,
+    uint32_t* rev_last,
+    cudaStream_t stream
+) {
+    if (rows <= 0 || rows > 65535 || cols <= 0 || cols > 32767 || !wmin || !wmax || wpitch < (size_t)cols || !fwd_last)
+        return cudaErrorInvalidValue;
+    note_search_kernel("windows<K=%d,flags=%d>", K, flags);
+    RangeArgs p {};
+    p.desc0 = desc0;
+    p.desc1 = desc1;
+    p.cols = cols;
+    p.pitch_words = desc_pitch_words;
+    // a CTA stages at most the whole row; the windows are only known on the device, so the chunk is the cap
+    const int cap = (RANGE_CHUNK_BYTES / (4 * K)) & ~3;
+    const int row4 = (cols + 3) & ~3;
+    p.chunk = row4 < cap ? row4 : cap;
+    p.fwd_first = fwd_first;
+    p.fwd_last = fwd_last;
+    p.rev_first = rev_first;
+    p.rev_last = rev_last;
+    p.wmin = wmin;
+    p.wmax = wmax;
+    p.wpitch = wpitch;
+    return launch_args<true>(p, K, rows, flags, stream);
 }
 
 } // namespace bicos_b200
